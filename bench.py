@@ -2,6 +2,7 @@
 """bench.py -- the hot path's headline metric on B200 (BASELINE.json): UTF-8 input GB/s (+ tokens/s) of batch encode.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mb MB] [--workload bpe|unigram|pipeline|mixed]
+                  [--dump-outputs DIR]
 
 One step = one pass of aksharTokenizer.encode over one batch: normalize_text -> BPE-24k ids for every row of the
 batch (BASELINE.json configs[1]: "BPE vocab 24k batch encode of 1 GB synthetic Hinglish, 1 B200").  Run without
@@ -17,6 +18,12 @@ batch API from pinned host buffers with the H2D copy of the text and the D2H rea
 SURVEY section 8d's bytes over the stage's kernels); `cpu_baseline` is the oracle port of the same path on the host cores
 (bounded sample) -- the same rows are compared id for id with the GPU's before anything is timed (`parity_in_run`).
 --impl reference times that CPU implementation alone, with every host core.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step returned as DIR/<workload>_<array>.npy (float32
+or float64, 64 MiB at most in all): for a fixed, seeded sample of rows their ids / normalized bytes / mask bits and
+their offsets into the full outputs, plus every batch's result counters.  The inputs depend only on the arguments, so two
+builds can be compared output for output.  Nothing is written into the source tree (not even bytecode): it may be
+read-only, and the library is the one __graft_entry__.build() left there.
 """
 import argparse
 import json
@@ -28,6 +35,7 @@ import threading
 import time
 import zlib
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, 'tools')):
     if p not in sys.path:
@@ -253,6 +261,67 @@ def traffic_table():
     return {}
 
 
+# ------------------------------------------------------------------ --dump-outputs
+DUMP_ROWS = 4096
+DUMP_LIMIT = 64 << 20
+
+
+def dump_rows(n_rows):
+    """the rows whose outputs are dumped: a fixed, seeded sample"""
+    import numpy as np
+    rng = np.random.default_rng(SEED)
+    return np.sort(rng.choice(n_rows, size=min(n_rows, DUMP_ROWS), replace=False))
+
+
+def _spans(lo, hi):
+    """flat indices lo[j] .. hi[j] - 1 of every j, concatenated"""
+    import numpy as np
+    n = hi - lo
+    return np.repeat(lo - np.cumsum(n) + n, n) + np.arange(int(n.sum()), dtype=np.int64)
+
+
+def sample_outputs(outs, ranges, rows, tokens):
+    """one step's per-batch outputs ((ids, normalized text, result) or (masks, normalized text, result)), restricted to the
+    rows `rows` (global indices) -> {name: float array}"""
+    import numpy as np
+    import torch
+    parts = {}
+    for (lo, hi), o in zip(ranges, outs):
+        norm = o[1]
+        dev = norm.offsets.device
+        t = torch.from_numpy(rows[(rows >= lo) & (rows < hi)] - lo).to(dev)
+        n0, n1 = norm.offsets[t].cpu().numpy(), norm.offsets[t + 1].cpu().numpy()
+        got = {'norm_offsets': np.stack([n0, n1], 1), 'norm': norm.data[torch.from_numpy(_spans(n0, n1)).to(dev)],
+               'result': o[-1][None]}
+        if tokens:
+            s0, s1 = o[0].splits[t].cpu().numpy(), o[0].splits[t + 1].cpu().numpy()
+            got['id_splits'] = np.stack([s0, s1], 1)
+            got['ids'] = o[0].values[torch.from_numpy(_spans(s0, s1)).to(dev)]
+        else:
+            # the four mask planes at every byte of a row and at its end (a cluster / run that ends a row sets the bit
+            # of the byte after it)
+            pos = torch.from_numpy(_spans(n0, n1 + 1)).to(dev)
+            planes = (o[0]['cluster'], o[0]['run'], o[0]['tags'][0], o[0]['tags'][1])
+            got['masks'] = torch.stack([(p[pos >> 5].to(torch.int64) >> (pos & 31)) & 1 for p in planes])
+        for k, v in got.items():
+            parts.setdefault(k, []).append(v.cpu().numpy() if torch.is_tensor(v) else v)
+    out = {k: np.concatenate(v, axis=-1) if k == 'masks' else np.concatenate(v) for k, v in parts.items()}
+    out['rows'] = rows
+    wide = ('norm_offsets', 'id_splits', 'result', 'rows')
+    return {k: v.astype(np.float64 if k in wide else np.float32) for k, v in out.items()}
+
+
+def write_dump(path, arrays):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError('--dump-outputs: %d bytes, more than %d' % (total, DUMP_LIMIT))
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), k
+        np.save(os.path.join(path, k + '.npy'), a)
+
+
 # ------------------------------------------------------------------ one workload on this rank
 class Rank:
     def __init__(self):
@@ -269,8 +338,9 @@ def describe(workload, mb, world):
                      'in 1 GiB batches' % (mb, world)}[workload]
 
 
-def run_workload(R, workload, mb, steps, warmup, cpu_sample_mb, dist, with_cpu=True):
-    """-> the JSON line (a dict) on rank 0, None elsewhere"""
+def run_workload(R, workload, mb, steps, warmup, cpu_sample_mb, dist, with_cpu=True, dump=None):
+    """-> the JSON line (a dict) on rank 0, None elsewhere; with `dump` (a dict) rank 0 adds the sampled outputs of the last
+    timed step to it"""
     import numpy as np
     import torch
     kind = KIND[workload]
@@ -404,11 +474,16 @@ def run_workload(R, workload, mb, steps, warmup, cpu_sample_mb, dist, with_cpu=T
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        device_step(dev_batches)
+        last = None             # a step's outputs are freed before the next step allocates, as if they were discarded
+        last = device_step(dev_batches)
     e1.record()
     barrier()
     launches = eng.launch_count() - l0
     ms = e0.elapsed_time(e1) / steps
+    if dump is not None and R.rank == 0:
+        for k, v in sample_outputs(last, ranges, dump_rows(n_rows), mkind is not None).items():
+            dump['%s_%s' % (workload, k)] = v
+    del last
 
     # ---- end to end through the public batch API: pinned host text in, ids (or offsets) on the host out
     bufs = {}
@@ -529,11 +604,12 @@ def run_workload(R, workload, mb, steps, warmup, cpu_sample_mb, dist, with_cpu=T
     }
 
 
-def config1_latency():
+def config1_latency(reps, dump=None):
     """BASELINE.json configs[0]: `aksharTokenizer().tokenize(line)` (no model: akshar-level fallback) over the reference's
     data/corpus.txt, one string per call -- the latency of the drop-in API (each call: pinned staging, two library calls,
     read-back), next to the same lines as ONE batch and to the CPU port of the same function on this box.  BASELINE.md
-    quotes 62 us/line for the reference's own Python path."""
+    quotes 62 us/line for the reference's own Python path.  With `dump`, the akshars of the last pass are added to it."""
+    import numpy as np
     import torch
     import akshar_b200 as A
     sys.path.insert(0, os.path.join(ROOT, 'oracle'))
@@ -543,13 +619,16 @@ def config1_latency():
     tk = A.aksharTokenizer()
     exp = [O.segment_akshars(O.normalize_text(s)) for s in lines]
     assert [tk.tokenize(s) for s in lines] == exp and tk.tokenize_batch(lines) == exp
-    reps = 20
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     for _ in range(reps):
-        for s in lines:
-            tk.tokenize(s)
+        last = [tk.tokenize(s) for s in lines]
     one = (time.perf_counter() - t0) / (reps * len(lines))
+    if dump is not None:
+        flat = [a for row in last for a in row]
+        dump['latency_akshars_per_line'] = np.array([len(row) for row in last], dtype=np.float64)
+        dump['latency_akshar_lengths'] = np.array([len(a) for a in flat], dtype=np.float64)
+        dump['latency_akshar_code_points'] = np.array([ord(c) for a in flat for c in a], dtype=np.float64)
     t0 = time.perf_counter()
     for _ in range(reps):
         tk.tokenize_batch(lines)
@@ -581,7 +660,12 @@ def main():
     ap.add_argument('--workload', default=None, choices=['bpe', 'unigram', 'pipeline', 'mixed'])
     ap.add_argument('--cpu-sample-mb', type=float, default=24.0)
     ap.add_argument('--no-also', action='store_true', help='headline workload only')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed (a seeded sample of rows) as DIR/<name>.npy')
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    dump = {} if a.dump_outputs else None
     R = Rank()
     workload = a.workload or ('bpe' if R.world == 1 else 'mixed')
     mb = a.mb or {'bpe': 1024, 'unigram': 1024, 'pipeline': 4096, 'mixed': 4096}[workload]
@@ -601,6 +685,10 @@ def main():
             tok += n
         native = arm.native_libs()
         arm.close()
+        if dump is not None:
+            import numpy as np
+            # what the CPU arm returns: one checksum of the reference's output per row of the sample
+            write_dump(a.dump_outputs, {'reference_%s_row_checksums' % workload: np.array(arm.sums, dtype=np.float64)})
         v = arm.nbytes * a.steps / t / 1e9
         metric = 'utf8_input_GBps_batch_encode' if workload != 'pipeline' else 'utf8_input_GBps_normalize_segment'
         print(json.dumps({
@@ -622,23 +710,22 @@ def main():
     if R.world > 1:
         import torch.distributed as dist
         dist.init_process_group('nccl', device_id=torch.device('cuda', R.local))
-    import __graft_entry__ as g
-    if R.rank == 0:
-        g.build()
-    if R.world > 1:
-        dist.barrier()
-    line = run_workload(R, workload, mb, a.steps, a.warmup, a.cpu_sample_mb, dist)
+    from akshar_b200 import _lib
+    _lib.load()                 # the library __graft_entry__.build() compiled; nothing is compiled here
+    line = run_workload(R, workload, mb, a.steps, a.warmup, a.cpu_sample_mb, dist, dump=dump)
     if a.workload is None and R.world == 1 and not a.no_also:
-        # BASELINE.json configs[2] and configs[3], measured the same way (fewer steps, smaller CPU samples)
+        # BASELINE.json configs[2] and configs[3], measured the same way (smaller CPU samples)
         import gc
         also = []
         for w, wmb in (('unigram', 1024), ('pipeline', 4096)):
             gc.collect()
             torch.cuda.empty_cache()
-            also.append(run_workload(R, w, wmb, min(a.steps, 3), 3, min(a.cpu_sample_mb, 8.0), dist))
-        also.append(config1_latency())
+            also.append(run_workload(R, w, wmb, a.steps, a.warmup, min(a.cpu_sample_mb, 8.0), dist, dump=dump))
+        also.append(config1_latency(a.steps, dump))
         line['also'] = also
     if R.rank == 0:
+        if dump is not None:
+            write_dump(a.dump_outputs, dump)
         print(json.dumps(line))
     if R.world > 1:
         dist.destroy_process_group()

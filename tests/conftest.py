@@ -51,3 +51,11 @@ def golden_raw():
     """vectors recorded from the unmodified reference with clean_hinglish=False (tools/make_golden_raw.py)"""
     with gzip.open(os.path.join(GOLDEN, 'reference_vectors_raw.json.gz'), 'rb') as f:
         return json.loads(f.read().decode('utf-8'))
+
+
+@pytest.fixture(scope='session')
+def library_fuzz():
+    """what the libraries the reference calls (unicodedata, regex, tokenizers, sentencepiece) returned for the wide-Unicode
+    fuzz rows (tools/make_golden_fuzz.py)"""
+    with gzip.open(os.path.join(GOLDEN, 'library_fuzz.json.gz'), 'rb') as f:
+        return json.loads(f.read().decode('utf-8'))

@@ -244,13 +244,11 @@ def test_zalgo_and_expanding_text():
     assert np.array_equal(grs, rs) and np.array_equal(gre, re_) and np.array_equal(grt, rt)
 
 
-def test_wide_unicode_fuzz():
-    """strings drawn from 38 blocks (combining marks, Hebrew / Arabic, nine Indic scripts, Hangul jamo and syllables,
-    compatibility ideographs, variation selectors, tags, flags, emoji ...): the oracle agrees with the libraries the
-    reference calls (unicodedata NFC, regex \\X), and walkers + bit-parallel lanes agree with the oracle"""
+def wide_unicode_lines():
+    """3000 strings drawn from 38 blocks (combining marks, Hebrew / Arabic, nine Indic scripts, Hangul jamo and syllables,
+    compatibility ideographs, variation selectors, tags, flags, emoji ...)"""
     import random
     import unicodedata as u
-    import regex
     rng = random.Random(2026)
     blocks = [(0x20, 0x7f), (0xa0, 0x17f), (0x300, 0x36f), (0x370, 0x3ff), (0x590, 0x5ff), (0x600, 0x6ff), (0x900, 0x97f),
               (0x980, 0x9ff), (0xa00, 0xa7f), (0xb80, 0xbff), (0xc00, 0xc7f), (0xd00, 0xd7f), (0xe00, 0xe7f), (0xf00, 0xfff),
@@ -273,8 +271,17 @@ def test_wide_unicode_fuzz():
         pool = [rcp() for _ in range(rng.choice((2, 4, 8)))]
         s = ''.join(rng.choice(pool) if rng.random() < 0.6 else rcp() for _ in range(n))
         lines.append(s.replace('\n', ' ').replace('\r', ' '))
-    assert all(O.normalize_unicode(s) == u.normalize('NFC', s) for s in lines)
-    assert all(O.segment_akshars(s) == regex.findall(r'\X', s) for s in lines)
+    return lines
+
+
+def test_wide_unicode_fuzz(library_fuzz):
+    """wide-Unicode strings: the oracle agrees with what the libraries the reference calls (unicodedata NFC, regex \\X)
+    returned for them (recorded by tools/make_golden_fuzz.py), and walkers + bit-parallel lanes agree with the oracle"""
+    lines = wide_unicode_lines()
+    ref = library_fuzz['walkers']
+    assert lines == ref['rows'], 'the generated rows are not the recorded ones'
+    assert [O.normalize_unicode(s) for s in lines] == ref['nfc']
+    assert [O.segment_akshars(s) for s in lines] == ref['clusters']
     data, off = sc.pack(lines)
     for flags, (nr, nc) in ((1, (True, False)), (7, (True, True)), (0, (False, False))):
         exp, exp_off = OB.normalize_batch(lines, nr, nc)

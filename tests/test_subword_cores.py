@@ -95,12 +95,13 @@ def test_signature_matches_reference(golden):
     assert got == [golden['signature'][w] for w in words]
 
 
-def test_loader_rejects_unsupported(models_dir):
+def test_loader_rejects_unsupported(models_dir, tmp_path):
     import json
     j = json.load(open(os.path.join(models_dir, 'bpe_corpus.json'), encoding='utf-8'))
     j['pre_tokenizer'] = {'type': 'ByteLevel'}
-    p = '/tmp/_ak_bad.json'
-    json.dump(j, open(p, 'w'))
+    p = str(tmp_path / 'bad.json')
+    with open(p, 'w') as f:
+        json.dump(j, f)
     with pytest.raises(ValueError):
         W.load_bpe(p)
     open(p, 'wb').write(b'\x00\x01garbage')
@@ -381,10 +382,9 @@ def test_zalgo_rows_through_the_event_stream_encoders(models_dir):
         assert st == 0 and np.array_equal(splits, sp) and ids.tolist() == flat
 
 
-def test_wide_unicode_fuzz_through_the_encoders(models_dir):
-    """rows drawn from 27 blocks (compatibility forms HF's NFKC rewrites, marks, Hangul, full-width forms, mathematical
-    alphanumerics, enclosed characters ...) with added-token syntax sprinkled in, `clean_hinglish=False`: the oracle gives
-    the ids of the libraries the reference calls (when they are installed), and the event-stream cores give the oracle's"""
+def wide_unicode_encoder_lines():
+    """1500 rows drawn from 27 blocks (compatibility forms HF's NFKC rewrites, marks, Hangul, full-width forms, mathematical
+    alphanumerics, enclosed characters ...) with added-token syntax sprinkled in, normalized with `clean_hinglish=False`"""
     import random
     import unicodedata as u
     rng = random.Random(77)
@@ -407,24 +407,21 @@ def test_wide_unicode_fuzz_through_the_encoders(models_dir):
         pool = [rcp() for _ in range(rng.choice((2, 4, 8)))] + [' ', '<s>', '</s>', '<unk>', '<']
         s = ''.join(rng.choice(pool) if rng.random() < 0.6 else rcp() for _ in range(n))
         lines.append(s.replace('\n', ' ').replace('\r', ' ').replace('\x00', ' '))
-    norm = [O.normalize_text(s, True, False) for s in lines]
+    return [O.normalize_text(s, True, False) for s in lines]
+
+
+def test_wide_unicode_fuzz_through_the_encoders(models_dir, library_fuzz):
+    """wide-Unicode rows: the oracle gives the ids the libraries the reference calls (tokenizers, sentencepiece) returned
+    for them (recorded by tools/make_golden_fuzz.py), and the event-stream cores give the oracle's"""
+    norm = wide_unicode_encoder_lines()
+    ref = library_fuzz['encoders']
+    assert norm == ref['rows'], 'the generated rows are not the recorded ones'
     mb = O.BpeModel(os.path.join(models_dir, 'bpe24k.json'))
     mu = O.UnigramModel(os.path.join(models_dir, 'spm24k.model'))
     exp_b = [O.bpe_encode(mb, s) for s in norm]
     exp_u = [O.unigram_encode(mu, s) for s in norm]
-    try:
-        from tokenizers import Tokenizer
-        tk = Tokenizer.from_file(os.path.join(models_dir, 'bpe24k.json'))
-        assert [tk.encode(s).ids for s in norm] == exp_b
-    except ImportError:
-        pass
-    try:
-        import sentencepiece as spm
-        sp = spm.SentencePieceProcessor()
-        sp.Load(os.path.join(models_dir, 'spm24k.model'))
-        assert [sp.EncodeAsIds(s) for s in norm] == exp_u
-    except ImportError:
-        pass
+    assert exp_b == ref['bpe24k']
+    assert exp_u == ref['spm24k']
     data, off = sc.pack(norm)
     W.load_bpe(os.path.join(models_dir, 'bpe24k.json'))
     ids, splits, st, _ = W.tok(0, data, off)

@@ -1,10 +1,11 @@
 #!/usr/bin/env python
 """What the words that are new in a call cost: the resolve kernel with the word cache restored at every call (default) and held."""
 import sys, os
-sys.path[:0]=['/root/repo','/root/repo/tools']
+ROOT=os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0]=[ROOT,os.path.join(ROOT,'tools')]
 import torch, akshar_b200 as A, synth_corpus as sc
 for what,kind,model,k in (('unigram','hindi','spm24k.model',1),('bpe','hinglish','bpe24k.json',0)):
-    tk=A.aksharTokenizer('/root/repo/tests/golden/models/'+model, 'sentencepiece' if k else 'bpe')
+    tk=A.aksharTokenizer(os.path.join(ROOT,'tests','golden','models',model), 'sentencepiece' if k else 'bpe')
     eng=tk._eng
     d,o=sc.Corpus(kind,20261018).generate(1<<30)
     b=eng.put((torch.from_numpy(d),torch.from_numpy(o)))

@@ -1,5 +1,6 @@
-import sys, time
-sys.path[:0]=['/root/repo','/root/repo/tools']
+import os, sys, time
+ROOT=os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0]=[ROOT,os.path.join(ROOT,'tools')]
 import torch, akshar_b200 as A, synth_corpus as sc
 eng=A.Engine(0)
 d,o=sc.Corpus('social',20261018).generate(1<<30)
