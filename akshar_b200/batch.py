@@ -93,6 +93,7 @@ class Engine:
             raise C.AksharCudaError('akshar_ctx_create: ' + msg)
         self._ws = None
         self._vocab = {}
+        self._pad = {}
 
     def __del__(self):
         try:
@@ -404,6 +405,90 @@ class Engine:
             return TextBatch(out, out_off, 0, total)
         raise BatchStatusError(bits, 'decode_batch (retries exhausted)')
 
+    # ------------------------------------------------------------------ ids -> model-ready windows
+    def pad_id(self, kind):
+        """id of the model's pad piece: the '<pad>' token of a BPE model, the '<pad>' control piece of a SentencePiece model
+        (which has none unless it was trained with pad_id >= 0); None without one"""
+        if kind not in self._pad:
+            want = 1 if kind == 0 else 3                          # BPE special token / SentencePiece CONTROL piece
+            self._pad[kind] = next((i for i, (p, t) in enumerate(self.vocab(kind)[1]) if p == '<pad>' and t == want), None)
+        return self._pad[kind]
+
+    def windows_batch(self, ids, kind, max_length=None, padding='longest', truncation=False, stride=0,
+                      return_overflowing_tokens=False, pad_to_multiple_of=None, padding_side='right', truncation_side='right',
+                      pad_id=None):
+        """encoder output -> the dense batch a model takes, bit-exact with HF tokenizers' truncation (with stride and
+        overflowing windows) and padding, and with what transformers' `tokenizer(texts, truncation=..., max_length=...,
+        stride=..., return_overflowing_tokens=..., padding=..., pad_to_multiple_of=..., return_tensors='pt')` returns
+        for the model's `<s> $A </s>` template (the rule: include/akshar_b200.h, akshar_windows_count).
+        ids: a Ragged of model `kind` from the encoders (int32 or uint16 values), or a (values, splits) pair.
+        padding: 'longest' (the longest window of the call) or 'max_length'; the width is then rounded up to
+        pad_to_multiple_of.  pad_id defaults to the model's pad piece.
+        -> dict of int64 device tensors: input_ids [N, L], attention_mask [N, L], and with return_overflowing_tokens
+        overflow_to_sample_mapping [N] (the row of every window; windows are in row order, window 0 first).
+        Raises ValueError where HF would misbehave (see the header) and for ids the encoder of this model did not produce.
+        One read-back of the result block (N, longest window, status); nothing else synchronises."""
+        values, splits = (ids.values, ids.splits) if isinstance(ids, Ragged) else ids
+        if padding not in ('longest', 'max_length'):
+            raise ValueError("padding must be 'longest' or 'max_length'")
+        if padding_side not in ('left', 'right') or truncation_side not in ('left', 'right'):
+            raise ValueError("padding_side and truncation_side must be 'left' or 'right'")
+        if (truncation or padding == 'max_length') and max_length is None:
+            raise ValueError('truncation and padding to max_length need max_length')
+        if not truncation and (stride or return_overflowing_tokens):
+            raise ValueError('stride and return_overflowing_tokens need truncation')
+        if pad_to_multiple_of is not None and pad_to_multiple_of < 1:
+            raise ValueError('pad_to_multiple_of must be positive')
+        if pad_id is None:
+            pad_id = self.pad_id(kind)
+            if pad_id is None:
+                raise ValueError('the model has no pad piece: pass pad_id')
+        dev = self.device
+        values, splits = values.to(dev), splits.to(dev, torch.int64)
+        if values.dtype not in (torch.int32, torch.uint16, torch.int16):
+            values = values.to(torch.int32)
+        if values.numel() >= 2 ** 31:
+            raise ValueError('windows_batch takes fewer than 2^31 ids per call')
+        u16 = 0 if values.dtype == torch.int32 else 1
+        n_rows = splits.numel() - 1
+        flags = ((C.WIN_TRUNCATE if truncation else 0) | (C.WIN_OVERFLOW if return_overflowing_tokens else 0) |
+                 (C.WIN_TRUNC_LEFT if truncation_side == 'left' else 0) | (C.WIN_PAD_LEFT if padding_side == 'left' else 0))
+        ml = max_length if max_length is not None else 0
+        need = self.lib.akshar_windows_workspace_bytes(n_rows)
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = None
+            self._ws = torch.empty(need + (need >> 3), dtype=torch.uint8, device=dev)
+        wsplits = torch.empty(n_rows + 1, dtype=torch.int64, device=dev)
+        result = torch.empty(4, dtype=torch.int64, device=dev)
+        rc = self.lib.akshar_windows_count(self._h, kind, values.data_ptr(), u16, splits.data_ptr(), n_rows, ml, stride, flags,
+                                           wsplits.data_ptr(), result.data_ptr(), self._ws.data_ptr(), self._ws.numel(), self._stream())
+        if rc == C.E_ARG:
+            raise ValueError(self.lib.akshar_last_error(self._h).decode())
+        if rc != 0:
+            self._err(rc, 'akshar_windows_count')
+        n, longest, bits = (int(x) for x in result.cpu()[:3])
+        if bits & C.ST_TEMPLATE:
+            raise ValueError('a row does not begin / end with the template ids of the model: not ids of its encoder')
+        if bits:
+            raise BatchStatusError(bits, 'windows_batch')
+        width = max_length if padding == 'max_length' else longest
+        if pad_to_multiple_of:
+            width = -(-width // pad_to_multiple_of) * pad_to_multiple_of
+        if longest > width:
+            raise ValueError('a row of %d ids is longer than max_length = %d: truncate it' % (longest, max_length))
+        out_ids = torch.empty((n, width), dtype=torch.int64, device=dev)
+        mask = torch.empty((n, width), dtype=torch.int64, device=dev)
+        sample = torch.empty(n, dtype=torch.int64, device=dev)
+        rc = self.lib.akshar_windows_write(self._h, kind, values.data_ptr(), u16, splits.data_ptr(), wsplits.data_ptr(), n_rows, n,
+                                           ml, stride, flags, width, pad_id, out_ids.data_ptr(), mask.data_ptr(), sample.data_ptr(),
+                                           self._stream())
+        if rc != 0:
+            self._err(rc, 'akshar_windows_write')
+        out = {'input_ids': out_ids, 'attention_mask': mask}
+        if return_overflowing_tokens:
+            out['overflow_to_sample_mapping'] = sample
+        return out
+
     def segment_masks(self, batch, clusters=True, matras=False, runs=False, out=None, check=True):
         """segment_batch with AKSHAR_SEG_MASK: the boundaries as bit masks, one bit per text byte (bit p - begin set when a
         cluster / run ends at byte p) -> dict(cluster=uint32 [W] | None, run=uint32 [W] | None, tags=uint32 [2, W] | None,
@@ -658,6 +743,7 @@ class Engine:
         if rc != 0:
             self._err(rc, 'akshar_load_bpe_json')
         self._vocab.pop(0, None)
+        self._pad.pop(0, None)
 
     def load_spm(self, path_or_bytes):
         """SentencePieceProcessor.Load for the CUDA path (reference tokenizer.py:88-91)"""
@@ -666,6 +752,7 @@ class Engine:
         if rc != 0:
             self._err(rc, 'akshar_load_spm_model')
         self._vocab.pop(1, None)
+        self._pad.pop(1, None)
 
     def vocab(self, kind):
         """[(token str, type)] by id; kind 0 BPE, 1 Unigram"""

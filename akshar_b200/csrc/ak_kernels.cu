@@ -38,6 +38,7 @@
 #include "ak_decode_kernels.cuh"
 #include "ak_feat_kernels.cuh"
 #include "ak_lines_kernels.cuh"
+#include "ak_win_kernels.cuh"
 
 // ================================================================================================
 // host side: context, model upload, C ABI

@@ -148,6 +148,16 @@ class aksharTokenizer:
             return ids, norm
         return [r.tolist() for r in ids.rows()]
 
+    def encode_batch_tensors(self, texts, **kwargs):
+        """encode() over a batch, returned as the dense tensors a model takes: encode_batch(as_device=True) followed by
+        Engine.windows_batch with the same keywords (max_length, padding, truncation, stride, return_overflowing_tokens,
+        pad_to_multiple_of, padding_side, truncation_side, pad_id) -> dict of int64 device tensors input_ids,
+        attention_mask (and overflow_to_sample_mapping), as transformers' tokenizer(texts, ..., return_tensors='pt')"""
+        if self.model is None:
+            raise ValueError("need model for IDs")
+        ids, _ = self.encode_batch(texts, as_device=True)
+        return self._eng.windows_batch(ids, self.model.kind, **kwargs)
+
     def encode_batch_host(self, h_data, h_offsets, out_ids=None, out_splits=None, compact=False):
         """encode() over a batch given as pinned host tensors (uint8 text, int64 row offsets) -> pinned host tensors
         (int32 ids, int64 row_splits), or with compact=True a `CompactIds` (uint16 ids, int32 chunk-relative splits: a third

@@ -57,6 +57,8 @@ enum {
     AKSHAR_ST_INTERNAL = 64,     /* an internal consistency check failed (never expected): the result is not to be used */
     AKSHAR_ST_BAD_ID = 128,      /* decode: a token id outside the vocabulary of a SentencePiece model (DecodeIds raises
                                     IndexError "piece id is out of range."); HF's decode skips such ids */
+    AKSHAR_ST_TEMPLATE = 256,    /* windows: a row does not begin with the template's bos / end with its eos (ids that the
+                                    encoder of this model did not produce) */
 };
 
 /* normalize flags: normalize_text(text, normalize_roman, clean_hinglish) (normalize.py:117) is
@@ -237,6 +239,40 @@ int akshar_tokenizer_encode_batch_ex(akshar_ctx* ctx, const uint8_t* d_text, con
                                      uint8_t* d_norm_text, int64_t norm_capacity, int64_t* d_norm_row_offsets, void* d_ids,
                                      int64_t id_capacity, void* d_id_splits, uint32_t out_flags, int64_t* d_result,
                                      void* d_workspace, size_t workspace_bytes, void* stream);
+
+/* Model-ready windows of encoder output, bit-exact with HF tokenizers' Tokenizer.enable_truncation(max_length, stride,
+ * direction) + enable_padding(direction, pad_id, length, pad_to_multiple_of) + encode_batch, flattened row by row as
+ * transformers flattens `[enc] + enc.overflowing` (return_overflowing_tokens=True).
+ * In: the ragged ids of one encoder call of model `kind` (0 BPE, 1 Unigram): d_ids int32 (or uint16 with ids_u16 != 0,
+ * the compact output of akshar_tokenizer_encode_batch_ex; may be NULL when the rows hold no ids), d_row_splits int64
+ * [n_rows + 1] positions in d_ids; fewer than 2^31 ids in one call.  The template ids s (2 for a BPE model whose post-processor is `<s> $A </s>`, 0 without one and
+ * for Unigram) come from the context's model; a row's content c is the row without them, m = max_length - s.
+ * Truncation (AKSHAR_WIN_TRUNCATE): a row with |c| <= m is one window; otherwise step = m - stride and window k is
+ * c[k step : min(k step + m, |c|)] (right) or c[max(|c| - k step - m, 0) : |c| - k step] (AKSHAR_WIN_TRUNC_LEFT) until a
+ * window reaches the end (start) of c: 1 + ceil((|c| - m) / step) windows; without AKSHAR_WIN_OVERFLOW only window 0.
+ * Every window is re-wrapped in the template ids.  Illegal values are refused with AKSHAR_E_ARG where HF misbehaves:
+ * max_length <= s, stride < 0 or >= m with truncation; stride != 0 or AKSHAR_WIN_OVERFLOW without it.
+ * Two calls:
+ *   akshar_windows_count: d_window_splits int64 [n_rows + 1] (window n belongs to row r for splits[r] <= n < splits[r + 1]);
+ *     result[0] = N windows, result[1] = longest window (template ids included), result[2] |= AKSHAR_ST_TEMPLATE when a
+ *     row is not framed by the template ids.
+ *   akshar_windows_write: for a width L >= the longest window (the caller picks it: the longest, or max_length, rounded up
+ *     to a multiple), d_input_ids / d_attention_mask int64 [n_windows, L] and d_sample int64 [n_windows] (the row of each
+ *     window: overflow_to_sample_mapping).  Pad positions hold pad_id and mask 0, on the right or on the left
+ *     (AKSHAR_WIN_PAD_LEFT); the other positions hold the window and mask 1.  n_windows, max_length, stride and flags are
+ *     those of the count call. */
+#define AKSHAR_WIN_TRUNCATE 1u
+#define AKSHAR_WIN_OVERFLOW 2u
+#define AKSHAR_WIN_TRUNC_LEFT 4u
+#define AKSHAR_WIN_PAD_LEFT 8u
+size_t akshar_windows_workspace_bytes(int64_t n_rows);
+int akshar_windows_count(akshar_ctx* ctx, int kind, const void* d_ids, int ids_u16, const int64_t* d_row_splits, int64_t n_rows,
+                         int64_t max_length, int64_t stride, uint32_t flags, int64_t* d_window_splits, int64_t* d_result,
+                         void* d_workspace, size_t workspace_bytes, void* stream);
+int akshar_windows_write(akshar_ctx* ctx, int kind, const void* d_ids, int ids_u16, const int64_t* d_row_splits,
+                         const int64_t* d_window_splits, int64_t n_rows, int64_t n_windows, int64_t max_length, int64_t stride,
+                         uint32_t flags, int64_t width, int64_t pad_id, int64_t* d_input_ids, int64_t* d_attention_mask,
+                         int64_t* d_sample, void* stream);
 
 /* Optional device-side timing of the dominant kernel of each stage, for roofline reporting: when enabled, the
  * library brackets that one launch with CUDA events on the caller's stream; akshar_timing_read waits for the
