@@ -11,7 +11,7 @@ LIB_PATH = os.environ.get('AKSHAR_B200_LIB') or os.path.join(_HERE, 'lib', 'liba
 
 OK, E_ARG, E_CUDA, E_MODEL, E_NOMODEL, E_WORKSPACE = 0, -1, -2, -3, -4, -5
 ST_OVERFLOW, ST_NFC_SEGMENT, ST_PATHOLOGICAL, ST_ALPHABET, ST_SPIN, ST_WORD, ST_INTERNAL, ST_BAD_ID = 1, 2, 4, 8, 16, 32, 64, 128
-ST_TEMPLATE = 256
+ST_TEMPLATE, ST_PAIR_TRUNC = 256, 512
 NORM_ROMAN, NORM_FILTER, NORM_COLLAPSE, NORM_CLEAN, NORM_NO_NFC = 1, 2, 4, 6, 8
 SEG_CLUSTERS, SEG_MATRAS, SEG_RUNS, SEG_MASK = 1, 2, 4, 8
 MODE_TILES, MODE_ROWS = 0, 1
@@ -19,7 +19,7 @@ OUT_IDS_U16, OUT_SPLITS_I32 = 1, 2
 WORDS_HINDI, WORDS_SPLIT = 0, 1
 FORM_DECODE, FORM_DETOKENIZE = 0, 1
 MERGE_AKSHARA, MERGE_NUKTA = 0, 1
-WIN_TRUNCATE, WIN_OVERFLOW, WIN_TRUNC_LEFT, WIN_PAD_LEFT = 1, 2, 4, 8
+WIN_TRUNCATE, WIN_OVERFLOW, WIN_TRUNC_LEFT, WIN_PAD_LEFT, WIN_ONLY_FIRST, WIN_ONLY_SECOND = 1, 2, 4, 8, 16, 32
 TIMERS = {'ak_nf3_classify_kernel': 0, 'ak_nf_write_kernel': 1, 'ak_resolve_kernel<bpe>': 2, 'ak_seg_off_kernel<emit>': 3, 'ak_seg_mask_kernel': 3,
           'ak_resolve_kernel<unigram>': 4, 'ak_words_kernel': 5, 'ak_emit_kernel': 6, 'ak_wtok_kernel': 7, 'ak_dec_kernel': 8, 'ak_lines_kernel': 9}
 
@@ -29,7 +29,8 @@ SYMBOLS = (
     'akshar_load_bpe_json', 'akshar_load_spm_model', 'akshar_vocab_size', 'akshar_vocab_token',
     'akshar_encode_bpe_batch', 'akshar_encode_unigram_batch', 'akshar_tokenizer_encode_batch', 'akshar_tokenizer_encode_batch_ex',
     'akshar_launch_count', 'akshar_timing_enable', 'akshar_timing_read', 'akshar_word_cache_hold', 'akshar_word_tokenize_batch', 'akshar_decode_workspace_bytes', 'akshar_decode_batch', 'akshar_composition_batch', 'akshar_merge_workspace_bytes', 'akshar_merge_clusters_batch', 'akshar_lines_workspace_bytes', 'akshar_lines_batch', 'akshar_join_rows', 'akshar_normalize_segment_batch',
-    'akshar_windows_workspace_bytes', 'akshar_windows_count', 'akshar_windows_write',
+    'akshar_windows_workspace_bytes', 'akshar_windows_count', 'akshar_windows_write', 'akshar_pair_windows_count',
+    'akshar_pair_windows_write',
 )
 
 _lib = None
@@ -81,6 +82,8 @@ def load():
     L.akshar_windows_workspace_bytes.restype = sz
     L.akshar_windows_count.argtypes = [vp, i32, vp, i32, vp, i64, i64, i64, u32, vp, vp, vp, sz, vp]
     L.akshar_windows_write.argtypes = [vp, i32, vp, i32, vp, vp, i64, i64, i64, i64, u32, i64, i64, vp, vp, vp, vp]
+    L.akshar_pair_windows_count.argtypes = [vp, i32, vp, vp, vp, vp, i32, i64, i64, i64, u32, vp, vp, vp, sz, vp]
+    L.akshar_pair_windows_write.argtypes = [vp, i32, vp, vp, vp, vp, i32, vp, i64, i64, i64, i64, u32, i64, i64, vp, vp, vp, vp]
     L.akshar_load_bpe_json.argtypes = [vp, c.c_char_p, sz]
     L.akshar_load_spm_model.argtypes = [vp, c.c_char_p, sz]
     L.akshar_vocab_size.argtypes = [vp, i32]

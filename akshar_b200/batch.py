@@ -48,6 +48,20 @@ class TextBatch:
         return [b[o[i]:o[i + 1]].decode('utf-8') for i in range(len(o) - 1)]
 
 
+# why akshar_pair_windows_count refused a pair (the reason in the low 3 bits of result[3])
+_PAIR_REFUSED = {1: 'longest_first would cut a sequence to 0 ids: max_length leaves 1 id for both',
+                 2: 'stride is not smaller than the length a sequence is cut to',
+                 3: 'sequence to truncate too short to respect the provided max_length',
+                 4: 'more than 2^31 - 1 windows'}
+
+
+def _ids_int32(v):
+    """int32 ids from int32 ids or compact ids (uint16, or the uint16 bit patterns an int16 tensor holds)"""
+    if v.dtype == torch.int16:
+        return v.to(torch.int32) & 0xFFFF
+    return v.to(torch.int32)
+
+
 class BatchStatusError(RuntimeError):
     def __init__(self, bits, what):
         self.bits = bits
@@ -416,7 +430,7 @@ class Engine:
 
     def windows_batch(self, ids, kind, max_length=None, padding='longest', truncation=False, stride=0,
                       return_overflowing_tokens=False, pad_to_multiple_of=None, padding_side='right', truncation_side='right',
-                      pad_id=None):
+                      pad_id=None, pair_ids=None):
         """encoder output -> the dense batch a model takes, bit-exact with HF tokenizers' truncation (with stride and
         overflowing windows) and padding, and with what transformers' `tokenizer(texts, truncation=..., max_length=...,
         stride=..., return_overflowing_tokens=..., padding=..., pad_to_multiple_of=..., return_tensors='pt')` returns
@@ -426,9 +440,21 @@ class Engine:
         pad_to_multiple_of.  pad_id defaults to the model's pad piece.
         -> dict of int64 device tensors: input_ids [N, L], attention_mask [N, L], and with return_overflowing_tokens
         overflow_to_sample_mapping [N] (the row of every window; windows are in row order, window 0 first).
+        pair_ids: the second sequences of sentence pairs (row i of ids with row i of pair_ids), as ids; the windows are
+        then those of `tokenizer(texts, text_pair, ...)` through the model's pair template (akshar_pair_windows_count),
+        and truncation takes True / 'longest_first', 'only_first', 'only_second', or False / 'do_not_truncate'.
         Raises ValueError where HF would misbehave (see the header) and for ids the encoder of this model did not produce.
         One read-back of the result block (N, longest window, status); nothing else synchronises."""
         values, splits = (ids.values, ids.splits) if isinstance(ids, Ragged) else ids
+        only = 0
+        if pair_ids is not None:
+            strategies = {'longest_first': 0, 'only_first': C.WIN_ONLY_FIRST, 'only_second': C.WIN_ONLY_SECOND}
+            if isinstance(truncation, str):
+                if truncation != 'do_not_truncate' and truncation not in strategies:
+                    raise ValueError("truncation must be True, False, 'longest_first', 'only_first', 'only_second' or "
+                                     "'do_not_truncate'")
+                only = strategies.get(truncation, 0)
+                truncation = truncation != 'do_not_truncate'
         if padding not in ('longest', 'max_length'):
             raise ValueError("padding must be 'longest' or 'max_length'")
         if padding_side not in ('left', 'right') or truncation_side not in ('left', 'right'):
@@ -447,12 +473,23 @@ class Engine:
         values, splits = values.to(dev), splits.to(dev, torch.int64)
         if values.dtype not in (torch.int32, torch.uint16, torch.int16):
             values = values.to(torch.int32)
+        if pair_ids is not None:
+            values_b, splits_b = (pair_ids.values, pair_ids.splits) if isinstance(pair_ids, Ragged) else pair_ids
+            values_b, splits_b = values_b.to(dev), splits_b.to(dev, torch.int64)
+            if values_b.dtype not in (torch.int32, torch.uint16, torch.int16):
+                values_b = values_b.to(torch.int32)
+            if (values.dtype == torch.int32) != (values_b.dtype == torch.int32):
+                values, values_b = _ids_int32(values), _ids_int32(values_b)
+            if splits_b.numel() != splits.numel():
+                raise ValueError('ids and pair_ids must hold the same number of rows')
+            if values_b.numel() >= 2 ** 31:
+                raise ValueError('windows_batch takes fewer than 2^31 ids per call')
         if values.numel() >= 2 ** 31:
             raise ValueError('windows_batch takes fewer than 2^31 ids per call')
         u16 = 0 if values.dtype == torch.int32 else 1
         n_rows = splits.numel() - 1
         flags = ((C.WIN_TRUNCATE if truncation else 0) | (C.WIN_OVERFLOW if return_overflowing_tokens else 0) |
-                 (C.WIN_TRUNC_LEFT if truncation_side == 'left' else 0) | (C.WIN_PAD_LEFT if padding_side == 'left' else 0))
+                 (C.WIN_TRUNC_LEFT if truncation_side == 'left' else 0) | (C.WIN_PAD_LEFT if padding_side == 'left' else 0) | only)
         ml = max_length if max_length is not None else 0
         need = self.lib.akshar_windows_workspace_bytes(n_rows)
         if self._ws is None or self._ws.numel() < need:
@@ -460,15 +497,25 @@ class Engine:
             self._ws = torch.empty(need + (need >> 3), dtype=torch.uint8, device=dev)
         wsplits = torch.empty(n_rows + 1, dtype=torch.int64, device=dev)
         result = torch.empty(4, dtype=torch.int64, device=dev)
-        rc = self.lib.akshar_windows_count(self._h, kind, values.data_ptr(), u16, splits.data_ptr(), n_rows, ml, stride, flags,
-                                           wsplits.data_ptr(), result.data_ptr(), self._ws.data_ptr(), self._ws.numel(), self._stream())
+        if pair_ids is None:
+            rc = self.lib.akshar_windows_count(self._h, kind, values.data_ptr(), u16, splits.data_ptr(), n_rows, ml, stride, flags,
+                                               wsplits.data_ptr(), result.data_ptr(), self._ws.data_ptr(), self._ws.numel(),
+                                               self._stream())
+        else:
+            rc = self.lib.akshar_pair_windows_count(self._h, kind, values.data_ptr(), splits.data_ptr(), values_b.data_ptr(),
+                                                    splits_b.data_ptr(), u16, n_rows, ml, stride, flags, wsplits.data_ptr(),
+                                                    result.data_ptr(), self._ws.data_ptr(), self._ws.numel(), self._stream())
         if rc == C.E_ARG:
             raise ValueError(self.lib.akshar_last_error(self._h).decode())
         if rc != 0:
-            self._err(rc, 'akshar_windows_count')
-        n, longest, bits = (int(x) for x in result.cpu()[:3])
+            self._err(rc, 'akshar_pair_windows_count' if pair_ids is not None else 'akshar_windows_count')
+        n, longest, bits, refused = (int(x) for x in result.cpu())
         if bits & C.ST_TEMPLATE:
             raise ValueError('a row does not begin / end with the template ids of the model: not ids of its encoder')
+        if bits & C.ST_PAIR_TRUNC:
+            if refused & 7 == 5:
+                raise ValueError('the %d pairs give more than 2^31 - 1 windows in all: window fewer pairs per call' % n_rows)
+            raise ValueError('pair %d: %s' % (refused >> 3, _PAIR_REFUSED.get(refused & 7, 'cannot be truncated as asked')))
         if bits:
             raise BatchStatusError(bits, 'windows_batch')
         width = max_length if padding == 'max_length' else longest
@@ -479,11 +526,16 @@ class Engine:
         out_ids = torch.empty((n, width), dtype=torch.int64, device=dev)
         mask = torch.empty((n, width), dtype=torch.int64, device=dev)
         sample = torch.empty(n, dtype=torch.int64, device=dev)
-        rc = self.lib.akshar_windows_write(self._h, kind, values.data_ptr(), u16, splits.data_ptr(), wsplits.data_ptr(), n_rows, n,
-                                           ml, stride, flags, width, pad_id, out_ids.data_ptr(), mask.data_ptr(), sample.data_ptr(),
-                                           self._stream())
+        if pair_ids is None:
+            rc = self.lib.akshar_windows_write(self._h, kind, values.data_ptr(), u16, splits.data_ptr(), wsplits.data_ptr(), n_rows,
+                                               n, ml, stride, flags, width, pad_id, out_ids.data_ptr(), mask.data_ptr(),
+                                               sample.data_ptr(), self._stream())
+        else:
+            rc = self.lib.akshar_pair_windows_write(self._h, kind, values.data_ptr(), splits.data_ptr(), values_b.data_ptr(),
+                                                    splits_b.data_ptr(), u16, wsplits.data_ptr(), n_rows, n, ml, stride, flags, width,
+                                                    pad_id, out_ids.data_ptr(), mask.data_ptr(), sample.data_ptr(), self._stream())
         if rc != 0:
-            self._err(rc, 'akshar_windows_write')
+            self._err(rc, 'akshar_pair_windows_write' if pair_ids is not None else 'akshar_windows_write')
         out = {'input_ids': out_ids, 'attention_mask': mask}
         if return_overflowing_tokens:
             out['overflow_to_sample_mapping'] = sample

@@ -39,6 +39,7 @@
 #include "ak_feat_kernels.cuh"
 #include "ak_lines_kernels.cuh"
 #include "ak_win_kernels.cuh"
+#include "ak_pair_kernels.cuh"
 
 // ================================================================================================
 // host side: context, model upload, C ABI

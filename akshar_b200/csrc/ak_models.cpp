@@ -352,6 +352,27 @@ std::string ak_parse_bpe_json(const char* json, size_t len, AkBpeHost& out) {
         if (seq_at + 1 < (int)single->arr.size() && !special_id(single->arr[(size_t)seq_at + 1], out.eos))
             return "unsupported TemplateProcessing layout";
         if (seq_at > 1) return "unsupported TemplateProcessing layout";
+        // `pre $A mid $B post` pair template: any other shape leaves the model usable for everything but pairs
+        const JVal* pair = pp->get("pair");
+        int slot = 0;
+        out.pair_ok = pair && pair->kind == JVal::Arr;
+        for (size_t i = 0; out.pair_ok && i < pair->arr.size(); ++i) {
+            const JVal& item = pair->arr[i];
+            const JVal* seq = item.get("Sequence");
+            int32_t id = -1;
+            if (seq) {
+                const JVal* nm_ = seq->get("id");
+                const char* want = slot == 0 ? "A" : "B";
+                out.pair_ok = slot < 2 && nm_ && nm_->kind == JVal::Str && nm_->str == want;
+                ++slot;
+            } else if (special_id(item, id) && out.pair_n[slot] < 4) {
+                out.pair_ids[slot][out.pair_n[slot]++] = id;
+            } else {
+                out.pair_ok = false;
+            }
+        }
+        if (slot != 2) out.pair_ok = false;
+        if (!out.pair_ok) out.pair_n[0] = out.pair_n[1] = out.pair_n[2] = 0;
     }
     return "";
 }

@@ -17,6 +17,11 @@ struct AkBpeHost {
     std::vector<unsigned long long> mkeys, mvals;  // open-addressing table, size 1 << mbits
     uint32_t mbits = 0;
     int32_t bos = -1, eos = -1;
+    // pair template `pre $A mid $B post` (post_processor.pair): the ids of each slot; pair_ok = false when the model has
+    // a pair template of another shape (then only the pair calls are refused)
+    int32_t pair_ids[3][4] = {};
+    int pair_n[3] = {0, 0, 0};
+    bool pair_ok = true;
     // added tokens (all `special`, matched in the raw text before the normalizer), longest first
     std::vector<uint8_t> sp_bytes;
     std::vector<uint16_t> sp_off;                  // [n + 1]

@@ -6,6 +6,7 @@
 //                          both outputs as coalesced int64 stores
 // The write is a gather: ids are read once per window position they land in, 16 bytes are written per output position.
 #pragma once
+#include "ak_win.cuh"
 
 #define AKWIN_THREADS 256
 
@@ -19,20 +20,6 @@ struct AkWinArgs {
     int64_t step;                      // m - stride
     bool overflow, left, pad_left;
 };
-
-// window k of a row with c content ids: [start, stop) in the content
-__device__ __forceinline__ void akwin_span(int64_t c, int64_t m, int64_t step, bool left, int64_t k, int64_t& start, int64_t& stop) {
-    if (c <= m) {
-        start = 0;
-        stop = c;
-    } else if (left) {
-        stop = c - k * step;
-        start = stop > m ? stop - m : 0;
-    } else {
-        start = k * step;
-        stop = start + m < c ? start + m : c;
-    }
-}
 
 // count[r] = windows of row r (count[n_rows] = 0, so that the scan's last entry is N); result[1] = longest window;
 // AKSHAR_ST_TEMPLATE when a row is not framed by the template ids
@@ -67,6 +54,25 @@ __global__ void __launch_bounds__(AKWIN_THREADS) ak_win_count_kernel(const AkWin
     }
 }
 
+// the row that owns window w, by the whole warp: the last r with wsplits[r] <= w (every row owns at least one window, so
+// the window splits increase strictly).  Lane i probes lo + 1 + i (hi - lo) / 32; the probes that pass form a prefix of
+// the lanes, so every step divides the range by 32
+__device__ __forceinline__ int64_t akwin_owner(const int64_t* __restrict__ wsplits, int64_t n_rows, int64_t w, int lane) {
+    int64_t lo = 0, hi = n_rows - 1;
+    while (lo < hi) {
+        const int64_t q = lo + 1 + ((hi - lo) * lane >> 5);
+        const unsigned pass = __ballot_sync(0xFFFFFFFFu, q <= hi && __ldg(wsplits + q) <= w);
+        const int last = 31 - __clz(pass | 1u);
+        const int64_t q_last = __shfl_sync(0xFFFFFFFFu, q, last), q_next = __shfl_sync(0xFFFFFFFFu, q, last < 31 ? last + 1 : 31);
+        if (!pass) hi = lo;
+        else {
+            hi = last < 31 ? q_next - 1 : hi;
+            lo = q_last;
+        }
+    }
+    return lo;
+}
+
 // one warp per window: the loads of AKWIN_UNROLL positions are issued before their stores (a load-store chain per
 // position leaves the warp waiting on every id), and the owning row is found by a 32-way search (log32 steps)
 #define AKWIN_UNROLL 8
@@ -78,21 +84,7 @@ __global__ void __launch_bounds__(AKWIN_THREADS) ak_win_write_kernel(const AkWin
     const int64_t warps = (int64_t)gridDim.x * (AKWIN_THREADS / 32);
     const int head = A.bos >= 0, s = head + (A.eos >= 0);
     for (int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n_windows; w += warps) {
-        // the row that owns window w: the last r with wsplits[r] <= w (every row owns at least one window, so the window
-        // splits increase strictly).  Lane i probes lo + 1 + i (hi - lo) / 32; the probes that pass form a prefix of the lanes
-        int64_t lo = 0, hi = A.n_rows - 1;
-        while (lo < hi) {
-            const int64_t q = lo + 1 + ((hi - lo) * lane >> 5);
-            const unsigned pass = __ballot_sync(0xFFFFFFFFu, q <= hi && __ldg(wsplits + q) <= w);
-            const int last = 31 - __clz(pass | 1u);
-            const int64_t q_last = __shfl_sync(0xFFFFFFFFu, q, last), q_next = __shfl_sync(0xFFFFFFFFu, q, last < 31 ? last + 1 : 31);
-            if (!pass) hi = lo;
-            else {
-                hi = last < 31 ? q_next - 1 : hi;
-                lo = q_last;
-            }
-        }
-        const int64_t r = lo, k = w - wsplits[r];
+        const int64_t r = akwin_owner(wsplits, A.n_rows, w, lane), k = w - wsplits[r];
         const int64_t r0 = A.splits[r], n = A.splits[r + 1] - r0;
         const int64_t c = n > s ? n - s : 0;
         int64_t start, stop;

@@ -148,15 +148,26 @@ class aksharTokenizer:
             return ids, norm
         return [r.tolist() for r in ids.rows()]
 
-    def encode_batch_tensors(self, texts, **kwargs):
+    def encode_batch_tensors(self, texts, text_pair=None, **kwargs):
         """encode() over a batch, returned as the dense tensors a model takes: encode_batch(as_device=True) followed by
         Engine.windows_batch with the same keywords (max_length, padding, truncation, stride, return_overflowing_tokens,
         pad_to_multiple_of, padding_side, truncation_side, pad_id) -> dict of int64 device tensors input_ids,
-        attention_mask (and overflow_to_sample_mapping), as transformers' tokenizer(texts, ..., return_tensors='pt')"""
+        attention_mask (and overflow_to_sample_mapping), as transformers' tokenizer(texts, ..., return_tensors='pt').
+        text_pair: the second texts of sentence pairs, as transformers' tokenizer(texts, text_pair, ...); texts and pairs
+        are encoded in one call and windowed through the model's pair template (truncation may then also be
+        'longest_first', 'only_first', 'only_second' or 'do_not_truncate')"""
         if self.model is None:
             raise ValueError("need model for IDs")
-        ids, _ = self.encode_batch(texts, as_device=True)
-        return self._eng.windows_batch(ids, self.model.kind, **kwargs)
+        if text_pair is None:
+            ids, _ = self.encode_batch(texts, as_device=True)
+            return self._eng.windows_batch(ids, self.model.kind, **kwargs)
+        texts, text_pair = list(texts), list(text_pair)
+        if len(texts) != len(text_pair):
+            raise ValueError('texts and text_pair must hold the same number of texts')
+        ids, _ = self.encode_batch(texts + text_pair, as_device=True)
+        n = len(texts)
+        return self._eng.windows_batch((ids.values, ids.splits[:n + 1]), self.model.kind,
+                                       pair_ids=(ids.values, ids.splits[n:]), **kwargs)
 
     def encode_batch_host(self, h_data, h_offsets, out_ids=None, out_splits=None, compact=False):
         """encode() over a batch given as pinned host tensors (uint8 text, int64 row offsets) -> pinned host tensors

@@ -59,6 +59,7 @@ enum {
                                     IndexError "piece id is out of range."); HF's decode skips such ids */
     AKSHAR_ST_TEMPLATE = 256,    /* windows: a row does not begin with the template's bos / end with its eos (ids that the
                                     encoder of this model did not produce) */
+    AKSHAR_ST_PAIR_TRUNC = 512,  /* pair windows: a pair cannot be truncated as asked (result[3] names it) */
 };
 
 /* normalize flags: normalize_text(text, normalize_roman, clean_hinglish) (normalize.py:117) is
@@ -273,6 +274,49 @@ int akshar_windows_write(akshar_ctx* ctx, int kind, const void* d_ids, int ids_u
                          const int64_t* d_window_splits, int64_t n_rows, int64_t n_windows, int64_t max_length, int64_t stride,
                          uint32_t flags, int64_t width, int64_t pad_id, int64_t* d_input_ids, int64_t* d_attention_mask,
                          int64_t* d_sample, void* stream);
+
+/* Model-ready windows of sentence pairs, bit-exact with HF tokenizers' Tokenizer.enable_truncation(max_length, stride,
+ * strategy, direction) + enable_padding(...) + encode_batch of (a, b) pairs through the model's TemplateProcessing
+ * pair template, flattened as transformers flattens `[enc] + enc.overflowing` (tokenizer(texts, text_pair, ...)).
+ * In: two ragged id sets of the encoder of model `kind`, one row per pair on each side: d_ids_a / d_splits_a [n_pairs + 1]
+ * and d_ids_b / d_splits_b [n_pairs + 1], int32 ids (uint16 with ids_u16 != 0, both sides); the two sides may share one
+ * ids buffer (texts and pairs encoded in one call: d_splits_b = d_splits_a + n_pairs).  Every row is framed by the
+ * single template as the encoder writes it; A and B are the rows without those ids, of ca and cb ids.
+ * The pair template is `pre $A mid $B post` (at most 4 ids per slot; the `<s> $A </s> <s> $B </s>` of a BPE model
+ * has P = |pre| + |mid| + |post| = 4; no post-processor and Unigram: P = 0); m = max_length - P.
+ * Truncation (AKSHAR_WIN_TRUNCATE; longest_first unless AKSHAR_WIN_ONLY_FIRST or AKSHAR_WIN_ONLY_SECOND):
+ *   1. ca + cb <= m: nothing is cut, one window.
+ *   2. else the lengths na, nb that A and B are cut to: longest_first: n1 = min(ca, cb); n2 = n1 if n1 > m, else
+ *      max(n1, m - n1); if n1 + n2 > m then n1 = m / 2 and n2 = n1 + m % 2; the larger goes to the longer sequence,
+ *      to B on a tie.  only_first / only_second: rem = ca + cb - m; the target sequence is cut to its length - rem.
+ *   3. a sequence that is cut (n < its length) has the windows of akshar_windows_count with m = n and the same
+ *      direction (AKSHAR_WIN_TRUNC_LEFT), wa windows for A and wb for B; a sequence not cut is one window.
+ *   4. with AKSHAR_WIN_OVERFLOW the pair gives wa * wb windows in the order (0, 0); (i, 0 .. wb - 1) for
+ *      i = 1 .. wa - 1; (0, j) for j = 1 .. wb - 1; without it only (0, 0).  Window (i, j) is pre + A_i + mid + B_j + post.
+ * Refused where HF misbehaves or raises: with AKSHAR_E_ARG for the call: m <= 0, stride < 0, stride > max_length - s
+ * with truncation (s: the single template's ids; HF's enable_truncation raises there, pairs or not), stride != 0 or
+ * AKSHAR_WIN_OVERFLOW without truncation, both ONLY flags, a model whose pair template is not of the form above
+ * ("unsupported pair template"); per pair, in result[2] |= AKSHAR_ST_PAIR_TRUNC and result[3] = the lowest
+ * pair * 8 + reason (1: longest_first would cut a sequence to 0 ids, 2: stride >= the length a sequence is cut to,
+ * 3: only_first / only_second and the target has no more than rem ids, 4: more than 2^31 - 1 windows); and for the
+ * whole call, when no pair is refused but the pairs give more than 2^31 - 1 windows in all, result[2] |=
+ * AKSHAR_ST_PAIR_TRUNC and result[3] = n_pairs * 8 + 5 (result[0] and d_window_splits are then not to be used).
+ * Two calls, as the single windows (workspace: akshar_windows_workspace_bytes(n_pairs)):
+ *   akshar_pair_windows_count: d_window_splits int64 [n_pairs + 1]; result[0] = N windows, result[1] = longest window
+ *     (always window (0, 0) of its pair), result[2] |= AKSHAR_ST_TEMPLATE when a row is not framed by the template ids.
+ *   akshar_pair_windows_write: d_input_ids / d_attention_mask int64 [n_windows, L] for a width L >= the longest window,
+ *     d_sample int64 [n_windows] (the pair of each window); pads as akshar_windows_write.  n_windows, max_length,
+ *     stride and flags are those of the count call. */
+#define AKSHAR_WIN_ONLY_FIRST 16u
+#define AKSHAR_WIN_ONLY_SECOND 32u
+int akshar_pair_windows_count(akshar_ctx* ctx, int kind, const void* d_ids_a, const int64_t* d_splits_a, const void* d_ids_b,
+                              const int64_t* d_splits_b, int ids_u16, int64_t n_pairs, int64_t max_length, int64_t stride,
+                              uint32_t flags, int64_t* d_window_splits, int64_t* d_result, void* d_workspace,
+                              size_t workspace_bytes, void* stream);
+int akshar_pair_windows_write(akshar_ctx* ctx, int kind, const void* d_ids_a, const int64_t* d_splits_a, const void* d_ids_b,
+                              const int64_t* d_splits_b, int ids_u16, const int64_t* d_window_splits, int64_t n_pairs,
+                              int64_t n_windows, int64_t max_length, int64_t stride, uint32_t flags, int64_t width,
+                              int64_t pad_id, int64_t* d_input_ids, int64_t* d_attention_mask, int64_t* d_sample, void* stream);
 
 /* Optional device-side timing of the dominant kernel of each stage, for roofline reporting: when enabled, the
  * library brackets that one launch with CUDA events on the caller's stream; akshar_timing_read waits for the
