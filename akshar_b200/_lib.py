@@ -11,7 +11,7 @@ LIB_PATH = os.environ.get('AKSHAR_B200_LIB') or os.path.join(_HERE, 'lib', 'liba
 
 OK, E_ARG, E_CUDA, E_MODEL, E_NOMODEL, E_WORKSPACE = 0, -1, -2, -3, -4, -5
 ST_OVERFLOW, ST_NFC_SEGMENT, ST_PATHOLOGICAL, ST_ALPHABET, ST_SPIN, ST_WORD, ST_INTERNAL, ST_BAD_ID = 1, 2, 4, 8, 16, 32, 64, 128
-ST_TEMPLATE, ST_PAIR_TRUNC = 256, 512
+ST_TEMPLATE, ST_PAIR_TRUNC, ST_PACK_LONG = 256, 512, 1024
 NORM_ROMAN, NORM_FILTER, NORM_COLLAPSE, NORM_CLEAN, NORM_NO_NFC = 1, 2, 4, 6, 8
 SEG_CLUSTERS, SEG_MATRAS, SEG_RUNS, SEG_MASK = 1, 2, 4, 8
 MODE_TILES, MODE_ROWS = 0, 1
@@ -30,7 +30,7 @@ SYMBOLS = (
     'akshar_encode_bpe_batch', 'akshar_encode_unigram_batch', 'akshar_tokenizer_encode_batch', 'akshar_tokenizer_encode_batch_ex',
     'akshar_launch_count', 'akshar_timing_enable', 'akshar_timing_read', 'akshar_word_cache_hold', 'akshar_word_tokenize_batch', 'akshar_decode_workspace_bytes', 'akshar_decode_batch', 'akshar_composition_batch', 'akshar_merge_workspace_bytes', 'akshar_merge_clusters_batch', 'akshar_lines_workspace_bytes', 'akshar_lines_batch', 'akshar_join_rows', 'akshar_normalize_segment_batch',
     'akshar_windows_workspace_bytes', 'akshar_windows_count', 'akshar_windows_write', 'akshar_pair_windows_count',
-    'akshar_pair_windows_write',
+    'akshar_pair_windows_write', 'akshar_pack_workspace_bytes', 'akshar_pack_count', 'akshar_pack_write',
 )
 
 _lib = None
@@ -84,6 +84,11 @@ def load():
     L.akshar_windows_write.argtypes = [vp, i32, vp, i32, vp, vp, i64, i64, i64, i64, u32, i64, i64, vp, vp, vp, vp]
     L.akshar_pair_windows_count.argtypes = [vp, i32, vp, vp, vp, vp, i32, i64, i64, i64, u32, vp, vp, vp, sz, vp]
     L.akshar_pair_windows_write.argtypes = [vp, i32, vp, vp, vp, vp, i32, vp, i64, i64, i64, i64, u32, i64, i64, vp, vp, vp, vp]
+    L.akshar_pack_workspace_bytes.argtypes = [i64]
+    L.akshar_pack_workspace_bytes.restype = sz
+    L.akshar_pack_count.argtypes = [vp, vp, i32, vp, i64, vp, vp, i64, i64, i64, vp, vp, sz, vp]
+    L.akshar_pack_write.argtypes = [vp, vp, i32, vp, i64, vp, vp, i64, i64, i64, i64, i64, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp,
+                                    sz, vp]
     L.akshar_load_bpe_json.argtypes = [vp, c.c_char_p, sz]
     L.akshar_load_spm_model.argtypes = [vp, c.c_char_p, sz]
     L.akshar_vocab_size.argtypes = [vp, i32]

@@ -541,6 +541,100 @@ class Engine:
             out['overflow_to_sample_mapping'] = sample
         return out
 
+    # ------------------------------------------------------------------ ids -> packed language-model batches
+    def pack_batch(self, ids, block_size, eos_id=None, carry=None, separator_id=-100, return_position_ids=True,
+                   return_seq_idx=False, return_flash_attn_kwargs=False):
+        """encoder output -> fixed blocks of `block_size` ids for causal-LM training without padding: the rows (one per
+        document, each followed by `eos_id` when one is given) concatenated after `carry` and cut into blocks as
+        transformers' run_clm.py `group_texts` cuts them, with the keys transformers'
+        DataCollatorWithFlattening(return_position_ids, separator_id, return_flash_attn_kwargs, return_seq_idx) returns
+        for the pieces the blocks and document starts cut the stream into (the rule: include/akshar_b200.h,
+        akshar_pack_count).  ids: a Ragged from the encoders (int32 or uint16 values), or a (values, splits) pair.
+        -> (batch, rest).  batch: input_ids, labels, position_ids (with return_position_ids) int64 [N, L] and seq_idx int32
+        [N, L] (with return_seq_idx); `.view(1, -1)` is the collator's layout, and with return_flash_attn_kwargs
+        cu_seq_lens_q / cu_seq_lens_k (int32 [pieces + 1], positions in that flattened layout) and max_length_q /
+        max_length_k (Python ints).  rest: the ids after the last whole block (fewer than block_size) as a device Ragged
+        (int32 values, int64 splits at document starts); pass it as the next call's `carry` and packing in chunks gives
+        the blocks of packing in one call.  Raises ValueError for block_size < 1, eos_id outside [0, 2^31), a carry not
+        of the returned form and a stream of 2^31 ids or more.  One read-back of the result block; nothing else
+        synchronises."""
+        if isinstance(block_size, bool) or not isinstance(block_size, int) or block_size < 1:
+            raise ValueError('block_size must be an int of at least 1')
+        if eos_id is not None and (isinstance(eos_id, bool) or not isinstance(eos_id, int) or not 0 <= eos_id < 2 ** 31):
+            raise ValueError('eos_id must be None or an int in [0, 2^31)')
+        if isinstance(separator_id, bool) or not isinstance(separator_id, int) or not -2 ** 63 <= separator_id < 2 ** 63:
+            raise ValueError('separator_id must be an int64')
+        dev = self.device
+        values, splits = (ids.values, ids.splits) if isinstance(ids, Ragged) else ids
+        values, splits = values.to(dev), splits.to(dev, torch.int64)
+        if values.dtype not in (torch.int32, torch.uint16, torch.int16):
+            values = values.to(torch.int32)
+        if splits.dim() != 1 or splits.numel() < 1:
+            raise ValueError('splits must be an int64 vector of n_rows + 1 positions')
+        if carry is None:
+            cv = cs = None
+            n_carry = 0
+        else:
+            if isinstance(carry, Ragged):
+                cv, cs = carry.values, carry.splits
+            elif isinstance(carry, (tuple, list)) and len(carry) == 2:
+                cv, cs = carry
+            else:
+                cv = cs = None
+            if not (isinstance(cv, torch.Tensor) and isinstance(cs, torch.Tensor) and cv.dtype == torch.int32 and
+                    cs.dtype == torch.int64 and cv.dim() == 1 and cs.dim() == 1 and cs.numel() >= 1 and cv.device == dev and
+                    cs.device == dev):
+                raise ValueError('carry must be the rest returned by pack_batch: (int32 values, int64 splits) on %s' % dev)
+            n_carry = cs.numel() - 1
+        if values.numel() + (cv.numel() if cv is not None else 0) >= 2 ** 31:
+            raise ValueError('pack_batch takes a stream of fewer than 2^31 ids per call (cu_seq_lens and seq_idx are int32)')
+        u16 = 0 if values.dtype == torch.int32 else 1
+        n_rows = splits.numel() - 1
+        eos = -1 if eos_id is None else eos_id
+        need = self.lib.akshar_pack_workspace_bytes(n_rows + n_carry)
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = None
+            self._ws = torch.empty(need + (need >> 3), dtype=torch.uint8, device=dev)
+        ws = self._ws
+        p = lambda t: t.data_ptr() if t is not None and t.numel() else None
+        args = (values.data_ptr() if values.numel() else None, u16, splits.data_ptr(), n_rows, p(cv), p(cs) if n_carry else None,
+                n_carry, block_size, eos)
+        result = torch.empty(8, dtype=torch.int64, device=dev)
+        rc = self.lib.akshar_pack_count(self._h, *args, result.data_ptr(), ws.data_ptr(), ws.numel(), self._stream())
+        if rc == C.E_ARG:
+            raise ValueError(self.lib.akshar_last_error(self._h).decode())
+        if rc != 0:
+            self._err(rc, 'akshar_pack_count')
+        n, n_pieces, bits, longest, total, n_frags, _, _ = (int(x) for x in result.cpu())
+        if bits & C.ST_PACK_LONG:
+            raise ValueError('the stream of this call holds %d ids: pack_batch takes fewer than 2^31 per call (cu_seq_lens '
+                             'and seq_idx are int32)' % total)
+        if bits:
+            raise BatchStatusError(bits, 'pack_batch')
+        L = block_size
+        out_ids = torch.empty((n, L), dtype=torch.int64, device=dev)
+        labels = torch.empty((n, L), dtype=torch.int64, device=dev)
+        pos = torch.empty((n, L), dtype=torch.int64, device=dev) if return_position_ids else None
+        seq = torch.empty((n, L), dtype=torch.int32, device=dev) if return_seq_idx else None
+        cu = torch.empty(n_pieces + 1, dtype=torch.int32, device=dev) if return_flash_attn_kwargs else None
+        rest_ids = torch.empty(total - n * L, dtype=torch.int32, device=dev)
+        rest_splits = torch.empty(n_frags + 1, dtype=torch.int64, device=dev)
+        q = lambda t: t.data_ptr() if t is not None else None
+        rc = self.lib.akshar_pack_write(self._h, *args, separator_id, total, n_pieces, n_frags, q(out_ids) if n else None,
+                                        q(labels) if n else None, q(pos) if n else None, q(seq) if n else None, q(cu),
+                                        p(rest_ids), rest_splits.data_ptr(), ws.data_ptr(), ws.numel(), self._stream())
+        if rc != 0:
+            self._err(rc, 'akshar_pack_write')
+        batch = {'input_ids': out_ids, 'labels': labels}
+        if return_position_ids:
+            batch['position_ids'] = pos
+        if return_seq_idx:
+            batch['seq_idx'] = seq
+        if return_flash_attn_kwargs:
+            batch['cu_seq_lens_q'] = batch['cu_seq_lens_k'] = cu
+            batch['max_length_q'] = batch['max_length_k'] = longest
+        return batch, Ragged(rest_ids, rest_splits)
+
     def segment_masks(self, batch, clusters=True, matras=False, runs=False, out=None, check=True):
         """segment_batch with AKSHAR_SEG_MASK: the boundaries as bit masks, one bit per text byte (bit p - begin set when a
         cluster / run ends at byte p) -> dict(cluster=uint32 [W] | None, run=uint32 [W] | None, tags=uint32 [2, W] | None,

@@ -182,3 +182,20 @@ def encode_lines(tokenizer, input_file, as_device=False, chunk_bytes=CHUNK_BYTES
         else:
             out.extend(r.tolist() for r in ids.rows())
     return out
+
+
+def pack_lines(tokenizer, input_file, block_size, chunk_bytes=CHUNK_BYTES, **kwargs):
+    """generator of packed causal-LM batches of a text file, one per piece of the file: every non-empty stripped line is
+    a document, encoded on the device and packed by Engine.pack_batch (keywords: eos_id, separator_id,
+    return_position_ids, return_seq_idx, return_flash_attn_kwargs).  The rest of each piece is the carry of the next,
+    so the blocks are those of packing the whole file in one call.  The ids after the file's last whole block are
+    dropped, as transformers' run_clm.py `group_texts` drops them."""
+    if tokenizer.model is None:
+        raise ValueError("need model for IDs")
+    if 'carry' in kwargs:
+        raise ValueError('pack_lines threads the carry itself')
+    carry = None
+    for rows in stream_rows(input_file, tokenizer._device, chunk_bytes):
+        ids, _ = tokenizer.encode_batch(rows, as_device=True)
+        batch, carry = tokenizer._eng.pack_batch(ids, block_size, carry=carry, **kwargs)
+        yield batch

@@ -40,6 +40,7 @@
 #include "ak_lines_kernels.cuh"
 #include "ak_win_kernels.cuh"
 #include "ak_pair_kernels.cuh"
+#include "ak_pack_kernels.cuh"
 
 // ================================================================================================
 // host side: context, model upload, C ABI

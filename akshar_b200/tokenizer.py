@@ -169,6 +169,17 @@ class aksharTokenizer:
         return self._eng.windows_batch((ids.values, ids.splits[:n + 1]), self.model.kind,
                                        pair_ids=(ids.values, ids.splits[n:]), **kwargs)
 
+    def encode_batch_packed(self, texts, block_size, **kwargs):
+        """encode() over a batch, packed into fixed blocks for causal-LM training: encode_batch(as_device=True) followed by
+        Engine.pack_batch with the same keywords (eos_id, carry, separator_id, return_position_ids, return_seq_idx,
+        return_flash_attn_kwargs) -> (batch, rest) as pack_batch returns them.  eos_id defaults to None: the rows of a
+        BPE model already end in its `</s>`, while SentencePiece rows carry neither `<s>` nor `</s>`, so SentencePiece
+        users pass the model's `</s>` id (2 for spm24k.model) to keep the documents of the stream apart."""
+        if self.model is None:
+            raise ValueError("need model for IDs")
+        ids, _ = self.encode_batch(texts, as_device=True)
+        return self._eng.pack_batch(ids, block_size, **kwargs)
+
     def encode_batch_host(self, h_data, h_offsets, out_ids=None, out_splits=None, compact=False):
         """encode() over a batch given as pinned host tensors (uint8 text, int64 row offsets) -> pinned host tensors
         (int32 ids, int64 row_splits), or with compact=True a `CompactIds` (uint16 ids, int32 chunk-relative splits: a third

@@ -60,6 +60,7 @@ enum {
     AKSHAR_ST_TEMPLATE = 256,    /* windows: a row does not begin with the template's bos / end with its eos (ids that the
                                     encoder of this model did not produce) */
     AKSHAR_ST_PAIR_TRUNC = 512,  /* pair windows: a pair cannot be truncated as asked (result[3] names it) */
+    AKSHAR_ST_PACK_LONG = 1024,  /* packed batches: the stream of the call holds 2^31 ids or more */
 };
 
 /* normalize flags: normalize_text(text, normalize_roman, clean_hinglish) (normalize.py:117) is
@@ -317,6 +318,40 @@ int akshar_pair_windows_write(akshar_ctx* ctx, int kind, const void* d_ids_a, co
                               const int64_t* d_splits_b, int ids_u16, const int64_t* d_window_splits, int64_t n_pairs,
                               int64_t n_windows, int64_t max_length, int64_t stride, uint32_t flags, int64_t width,
                               int64_t pad_id, int64_t* d_input_ids, int64_t* d_attention_mask, int64_t* d_sample, void* stream);
+
+/* Packed language-model batches: the rows of one call concatenated into one stream and cut into blocks of L ids, as
+ * transformers' run_clm.py `group_texts` does, with what a padding-free model needs to keep the documents apart, as
+ * transformers' DataCollatorWithFlattening(return_flash_attn_kwargs=True, return_seq_idx=True) returns it.
+ * In: ragged rows of ids, one per document (d_ids int32, or uint16 with ids_u16 != 0; d_row_splits int64 [n_rows + 1]),
+ * block_size L >= 1, eos_id in [0, 2^31) or -1 for none, and a carry: the rest of the previous call (d_carry int32 ids,
+ * d_carry_splits int64 [n_carry + 1]; n_carry = 0 and NULL pointers for none).
+ *   1. Stream S: the carry's fragments verbatim, then every row's ids, each followed by eos_id when one is given.  A
+ *      document start is the start of a non-empty fragment or row (an empty row adds nothing without eos_id, and the
+ *      document [eos] with it).  Unit u (fragment u, then row u - n_carry) starts at s_u = carry_splits[u] -
+ *      carry_splits[0], or C + (splits[r] - splits[0]) + (eos ? r : 0) for row r, C the carry's ids.
+ *   2. T = |S| < 2^31, N = T / L; block b is S[b L : (b + 1) L].  The rest S[N L : T] (< L ids) is returned in the carry's
+ *      form, its fragments split at document starts; passed as the next call's carry, packing in chunks equals packing
+ *      in one call.
+ *   3. Pieces start at every block start and every document start below N L.  Position p < N L of the document that
+ *      starts at s: position_ids = p - max(s, (p / L) L); labels = separator_id where position_ids = 0, else S[p];
+ *      seq_idx = the index of p's piece; cu_seq_lens = the piece starts, then N L; the longest piece is max_length.
+ * Refused with AKSHAR_E_ARG: L < 1, eos_id outside [0, 2^31) and not -1, more than 2^29 - 1 rows or fragments; and on
+ * the device with result[2] |= AKSHAR_ST_PACK_LONG: a stream of 2^31 ids or more (cu_seq_lens and seq_idx are int32).
+ * Two calls (workspace: akshar_pack_workspace_bytes(n_rows + n_carry), the same for both and kept between them):
+ *   akshar_pack_count: d_result int64 [8]: [0] N, [1] P pieces, [2] status, [3] longest piece, [4] T, [5] F fragments of
+ *     the rest, [6..7] 0.  Read back once; every size below follows from it.
+ *   akshar_pack_write, with T, P and F of the count call: d_input_ids and d_labels int64 [N L]; d_position_ids int64
+ *     [N L], d_seq_idx int32 [N L] and d_cu_seq_lens int32 [P + 1], each NULL when not wanted; d_rest_ids int32
+ *     [T - N L] and d_rest_splits int64 [F + 1] (always).  The other arguments are those of the count call. */
+size_t akshar_pack_workspace_bytes(int64_t n_units);
+int akshar_pack_count(akshar_ctx* ctx, const void* d_ids, int ids_u16, const int64_t* d_row_splits, int64_t n_rows,
+                      const int32_t* d_carry, const int64_t* d_carry_splits, int64_t n_carry, int64_t block_size, int64_t eos_id,
+                      int64_t* d_result, void* d_workspace, size_t workspace_bytes, void* stream);
+int akshar_pack_write(akshar_ctx* ctx, const void* d_ids, int ids_u16, const int64_t* d_row_splits, int64_t n_rows,
+                      const int32_t* d_carry, const int64_t* d_carry_splits, int64_t n_carry, int64_t block_size, int64_t eos_id,
+                      int64_t separator_id, int64_t total, int64_t n_pieces, int64_t n_rest_fragments, int64_t* d_input_ids,
+                      int64_t* d_labels, int64_t* d_position_ids, int32_t* d_seq_idx, int32_t* d_cu_seq_lens,
+                      int32_t* d_rest_ids, int64_t* d_rest_splits, void* d_workspace, size_t workspace_bytes, void* stream);
 
 /* Optional device-side timing of the dominant kernel of each stage, for roofline reporting: when enabled, the
  * library brackets that one launch with CUDA events on the caller's stream; akshar_timing_read waits for the
