@@ -28,7 +28,7 @@ SYMBOLS = (
     'akshar_workspace_bytes', 'akshar_normalize_batch', 'akshar_segment_batch', 'akshar_signature_batch',
     'akshar_load_bpe_json', 'akshar_load_spm_model', 'akshar_vocab_size', 'akshar_vocab_token',
     'akshar_encode_bpe_batch', 'akshar_encode_unigram_batch', 'akshar_tokenizer_encode_batch', 'akshar_tokenizer_encode_batch_ex',
-    'akshar_launch_count', 'akshar_timing_enable', 'akshar_timing_read', 'akshar_word_cache_hold', 'akshar_word_tokenize_batch', 'akshar_decode_workspace_bytes', 'akshar_decode_batch', 'akshar_composition_batch', 'akshar_merge_workspace_bytes', 'akshar_merge_clusters_batch', 'akshar_lines_workspace_bytes', 'akshar_lines_batch', 'akshar_join_rows', 'akshar_normalize_segment_batch',
+    'akshar_launch_count', 'akshar_timing_enable', 'akshar_timing_read', 'akshar_word_cache_hold', 'akshar_word_cache_stats', 'akshar_word_tokenize_batch', 'akshar_decode_workspace_bytes', 'akshar_decode_batch', 'akshar_composition_batch', 'akshar_merge_workspace_bytes', 'akshar_merge_clusters_batch', 'akshar_lines_workspace_bytes', 'akshar_lines_batch', 'akshar_join_rows', 'akshar_normalize_segment_batch',
     'akshar_windows_workspace_bytes', 'akshar_windows_count', 'akshar_windows_write', 'akshar_pair_windows_count',
     'akshar_pair_windows_write', 'akshar_pack_workspace_bytes', 'akshar_pack_count', 'akshar_pack_write',
 )
@@ -99,6 +99,7 @@ def load():
     L.akshar_tokenizer_encode_batch_ex.argtypes = [vp, vp, vp, i64, i64, i64, u32, i32, i32, vp, i64, vp, vp, i64, vp, u32, vp, vp, sz, vp]
     L.akshar_timing_enable.argtypes = [vp, i32]
     L.akshar_word_cache_hold.argtypes = [vp, i32]
+    L.akshar_word_cache_stats.argtypes = [vp, i32, vp, vp]
     L.akshar_timing_read.argtypes = [vp, i32, c.POINTER(c.c_float)]
     L.akshar_launch_count.argtypes = [vp]
     L.akshar_launch_count.restype = i64

@@ -805,6 +805,9 @@ class Engine:
                 if bits:
                     # this chunk again through the plain path (larger capacities / the row-sequential normalizer)
                     self.redone_chunks = getattr(self, 'redone_chunks', 0) + 1
+                    # the plain path uses the engine's one workspace, which chunks k + 1 and k + 2 are still using on
+                    # s_comp: start it after them (its read-back then ends it before chunk k + 3)
+                    s_out.wait_stream(s_comp)
                     b0, b1 = int(off_np[lo]), int(off_np[hi])
                     nbatch, mk = self.normalize_segment_batch((h_data[b0:b1], h_off[lo:hi + 1] - b0), normalize_roman, clean_hinglish,
                                                               True, matras, True)
@@ -1127,6 +1130,9 @@ class Engine:
                 d_ids, d_sp = S['ids'], S['splits']
                 if bits:
                     self.redone_chunks = getattr(self, 'redone_chunks', 0) + 1
+                    # the plain path uses the engine's one workspace and the model's word cache, which chunks k + 1 and
+                    # k + 2 are still using on s_comp: start it after them (its read-back then ends it before chunk k + 3)
+                    s_out.wait_stream(s_comp)
                     d_ids, d_sp, n = redo_chunk(k)
                 if state['tok'] + n > out_ids.numel():
                     if own_ids:

@@ -49,6 +49,7 @@ struct AkcTable {
     AkWordCache work{};
     unsigned long long* image = nullptr;
     size_t bytes = 0;
+    int64_t image_entries = 0;     // entries of the image built at load
     bool reset = false;            // restore the image at the next call whatever the fill
 };
 
@@ -208,6 +209,22 @@ int akshar_word_cache_hold(akshar_ctx* ctx, int hold) {
         return AKSHAR_OK;
     }
     ctx->wc_hold = hold != 0;
+    return AKSHAR_OK;
+}
+
+int akshar_word_cache_stats(akshar_ctx* ctx, int kind, int64_t* out, void* stream) {
+    if (!ctx || !out || (kind != 0 && kind != 1)) return AKSHAR_E_ARG;
+    // the Unigram encoder has a word cache only with the word-wise model shape
+    if (kind == 0 ? !ctx->has_bpe : !(ctx->has_uni && ctx->uni_fast)) return AKSHAR_E_NOMODEL;
+    AkDeviceGuard device_guard(ctx->device);
+    const AkcTable& t = ctx->tok_cache[kind];
+    unsigned long long learned = 0;
+    AK_CUDA(ctx, cudaMemcpyAsync(&learned, t.work.inserted, sizeof(learned), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    AK_CUDA(ctx, cudaStreamSynchronize((cudaStream_t)stream));
+    out[0] = (int64_t)1 << t.work.bits;
+    out[1] = t.image_entries;
+    out[2] = (int64_t)learned;
+    out[3] = ctx->wc_hold ? 1 : 0;
     return AKSHAR_OK;
 }
 

@@ -12,7 +12,8 @@
  *   - ragged outputs: values + `row_splits[n_rows + 1]` (int64).  Capacities are in elements; writes beyond a
  *     capacity are dropped, totals stay exact and AKSHAR_ST_OVERFLOW is raised in the result block.
  *   - `d_result` is 4 x int64 in device memory: [0] primary total, [1] secondary total, [2] status bits, [3] 0 (encoders
- *     that raise AKSHAR_ST_OVERFLOW for want of event slots: the slots per 960 text bytes that were needed).
+ *     that raise AKSHAR_ST_OVERFLOW for want of event slots: the slots per 960 text bytes that were needed; the id
+ *     total of akshar_tokenizer_encode_batch is then 0, as it is when its normalize stage overflowed).
  *   - return value: 0 on success, negative AKSHAR_E_* for host-side errors (bad argument, CUDA launch failure).
  *   - one context per device; a context is not thread-safe.
  */
@@ -378,6 +379,12 @@ int akshar_timing_enable(akshar_ctx* ctx, int enable);
  * next call (decided on the device).  hold = 1 switches that restore off, hold = 0 (default) on again, hold < 0
  * restores the image at the next encode call whatever the fill. */
 int akshar_word_cache_hold(akshar_ctx* ctx, int hold);
+/* Read-only state of the word cache of model `kind` (0 BPE, 1 Unigram), for tests and monitoring: out[0] = slots of the
+ * table, out[1] = entries of the image built at load, out[2] = entries learned since the last restore (read on `stream`,
+ * which is then synchronised), out[3] = the context's hold flag.  Only a restore empties a slot, so out[1] + out[2] slots
+ * are occupied.  AKSHAR_E_NOMODEL when the model is not loaded or has no word cache (a Unigram model without the
+ * word-wise shape). */
+int akshar_word_cache_stats(akshar_ctx* ctx, int kind, int64_t* out, void* stream);
 int akshar_timing_read(akshar_ctx* ctx, int timer, float* ms);
 
 /* number of kernels this library has launched on this context since creation (bench.py's gpu_launches) */
