@@ -122,20 +122,23 @@ class Engine:
         raise C.AksharCudaError('%s: %s (%s)' % (what, self.lib.akshar_status_str(rc).decode(),
                                                  self.lib.akshar_last_error(self._h).decode()))
 
-    def _workspace(self, n_bytes, n_rows, extra=0):
-        """`extra` bytes beyond the library's minimum enlarge the temporary output streams (grown after an overflow)"""
-        need = self.lib.akshar_workspace_bytes(n_bytes, n_rows) + extra
+    def _grow_ws(self, need):
+        """the engine's one workspace, of at least `need` bytes: it only grows, by an eighth more than asked, and the old
+        tensor is dropped before the new one is allocated"""
         if self._ws is None or self._ws.numel() < need:
             self._ws = None
             self._ws = torch.empty(need + (need >> 3), dtype=torch.uint8, device=self.device)
         return self._ws
 
+    def _workspace(self, n_bytes, n_rows, extra=0):
+        """`extra` bytes beyond the library's minimum enlarge the temporary output streams (grown after an overflow)"""
+        return self._grow_ws(self.lib.akshar_workspace_bytes(n_bytes, n_rows) + extra)
+
     MAX_TRIES = 5
 
-    def _slot_extra(self, n_bytes):
-        """workspace beyond the minimum that gives every 960-byte warp tile the event slots the last call asked for
+    def _slot_extra(self, n_bytes, need):
+        """workspace beyond the minimum that gives every 960-byte warp tile the `need` event slots an encoder call asked for
         (half of a surplus goes to the slots, 20 bytes each; include/akshar_b200.h)"""
-        need = getattr(self, '_slots_needed', 0)
         if need <= 256:
             return 0
         cap = 512
@@ -191,19 +194,28 @@ class Engine:
             self._stage_ev.record(torch.cuda.current_stream(self.device))
         return TextBatch(d, o, int(off[0]), int(off[-1]))
 
-    def _finish(self, result, what, check):
-        if not check:
-            return None
-        r = result.cpu()
-        bits = int(r[2])
-        self._slots_needed = int(r[3])        # encoders: event slots per 960 text bytes that were needed (on overflow)
-        return int(r[0]), int(r[1]), bits
+    def _finish(self, result):
+        """the result block read back: [0] primary total, [1] secondary total, [2] status bits, [3] call-specific"""
+        return tuple(int(x) for x in result.cpu())
+
+    def _ids_in(self, ids):
+        """ids from the encoders as a Ragged or a (values, splits) pair -> (values, int64 splits, u16) on this engine's
+        device; values that are neither int32 nor compact (uint16, or the uint16 bit patterns of int16) become int32"""
+        values, splits = (ids.values, ids.splits) if isinstance(ids, Ragged) else ids
+        values, splits = values.to(self.device), splits.to(self.device, torch.int64)
+        if values.dtype not in (torch.int32, torch.uint16, torch.int16):
+            values = values.to(torch.int32)
+        return values, splits, 0 if values.dtype == torch.int32 else 1
 
     # ------------------------------------------------------------------ K1
     def normalize_batch(self, batch, normalize_roman=True, clean_hinglish=True, mode=C.MODE_TILES, capacity=None, check=True):
         """normalize_text over a batch (reference normalize.py:117-148) -> TextBatch"""
-        b = self.put(batch)
         flags = (C.NORM_ROMAN if normalize_roman else 0) | (C.NORM_CLEAN if clean_hinglish else 0)
+        return self._normalize(batch, flags, mode, capacity, check)
+
+    def _normalize(self, batch, flags, mode=C.MODE_TILES, capacity=None, check=True):
+        """normalize_batch with AKSHAR_NORM_* flags as they are (the stand-alone stages of normalize.py)"""
+        b = self.put(batch)
         cap = capacity if capacity is not None else b.n_bytes + (b.n_bytes >> 3) + 1024
         ws = self._workspace(b.n_bytes, b.n_rows)
         for _ in range(self.MAX_TRIES):
@@ -217,7 +229,7 @@ class Engine:
                 self._err(rc, 'akshar_normalize_batch')
             if not check:
                 return TextBatch(out, out_off, 0, -1), result
-            total, _, bits = self._finish(result, 'normalize', True)
+            total, _, bits, _ = self._finish(result)
             if bits & C.ST_PATHOLOGICAL and mode == C.MODE_TILES:
                 mode = C.MODE_ROWS
                 continue
@@ -256,7 +268,7 @@ class Engine:
             if rc != 0:
                 self._err(rc, 'akshar_segment_batch')
             if check:
-                nc, nr, bits = self._finish(result, 'segment', True)
+                nc, nr, bits, _ = self._finish(result)
                 if bits & C.ST_PATHOLOGICAL and mode == C.MODE_TILES:
                     mode = C.MODE_ROWS
                     continue
@@ -298,7 +310,7 @@ class Engine:
                                                      ws.numel(), self._stream())
             if rc != 0:
                 self._err(rc, 'akshar_word_tokenize_batch')
-            total, _, bits = self._finish(result, 'word_tokenize', True)
+            total, _, bits, _ = self._finish(result)
             if bits & C.ST_OVERFLOW:
                 cap = total
                 continue
@@ -315,11 +327,7 @@ class Engine:
         dev = self.device
         rcap = row_capacity if row_capacity is not None else n_bytes // 24 + 1024
         for _ in range(self.MAX_TRIES):
-            need = self.lib.akshar_lines_workspace_bytes(n_bytes, rcap)
-            if self._ws is None or self._ws.numel() < need:
-                self._ws = None
-                self._ws = torch.empty(need + (need >> 3), dtype=torch.uint8, device=dev)
-            ws = self._ws
+            ws = self._grow_ws(self.lib.akshar_lines_workspace_bytes(n_bytes, rcap))
             out = torch.empty(max(n_bytes, 1), dtype=torch.uint8, device=dev)
             off = torch.empty(rcap + 1, dtype=torch.int64, device=dev)
             result = torch.empty(4, dtype=torch.int64, device=dev)
@@ -327,8 +335,7 @@ class Engine:
                                              result.data_ptr(), ws.data_ptr(), ws.numel(), self._stream())
             if rc != 0:
                 self._err(rc, 'akshar_lines_batch')
-            r = result.cpu()
-            rows, total, bits = int(r[0]), int(r[1]), int(r[2])
+            rows, total, bits, _ = self._finish(result)
             if bits & C.ST_OVERFLOW:
                 rcap = rows
                 continue
@@ -363,11 +370,7 @@ class Engine:
         """the cluster-merging feature wrappers (reference features.py:28-55, 173-206) -> Ragged like `clusters`"""
         b = self.put(batch)
         n = clusters.values.numel()
-        need = self.lib.akshar_merge_workspace_bytes(n)
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = None
-            self._ws = torch.empty(need + (need >> 3), dtype=torch.uint8, device=self.device)
-        ws = self._ws
+        ws = self._grow_ws(self.lib.akshar_merge_workspace_bytes(n))
         out = torch.empty(max(n, 1), dtype=torch.int32, device=self.device)
         sp = torch.empty(b.n_rows + 1, dtype=torch.int64, device=self.device)
         result = torch.empty(4, dtype=torch.int64, device=self.device)
@@ -376,7 +379,7 @@ class Engine:
                                                   result.data_ptr(), ws.data_ptr(), ws.numel(), self._stream())
         if rc != 0:
             self._err(rc, 'akshar_merge_clusters_batch')
-        total, _, bits = self._finish(result, 'merge_clusters', True)
+        total, _, bits, _ = self._finish(result)
         if bits:
             raise BatchStatusError(bits, 'merge_clusters_batch')
         return Ragged(out[:total], sp)
@@ -385,30 +388,21 @@ class Engine:
     def decode_batch(self, ids, splits, kind, form=C.FORM_DECODE, capacity=None):
         """aksharTokenizer.decode / detokenize over a batch of id rows (reference tokenizer.py:195-246) -> TextBatch.
         ids: device int32 (or uint16) tensor, or a Ragged from encode; splits: int64 [n_rows + 1] positions in ids"""
-        if isinstance(ids, Ragged):
-            ids, splits = ids.values, ids.splits
+        ids, splits, u16 = self._ids_in(ids if isinstance(ids, Ragged) else (ids, splits))
         dev = self.device
-        ids = ids.to(dev)
-        splits = splits.to(dev)
-        if ids.dtype not in (torch.int32, torch.uint16, torch.int16):
-            ids = ids.to(torch.int32)
         n_ids, n_rows = ids.numel(), splits.numel() - 1
-        need = self.lib.akshar_decode_workspace_bytes(n_ids, n_rows)
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = None
-            self._ws = torch.empty(need + (need >> 3), dtype=torch.uint8, device=dev)
-        ws = self._ws
+        ws = self._grow_ws(self.lib.akshar_decode_workspace_bytes(n_ids, n_rows))
         cap = capacity if capacity is not None else 6 * n_ids + 1024
         for _ in range(self.MAX_TRIES):
             out = torch.empty(max(cap, 1), dtype=torch.uint8, device=dev)
             out_off = torch.empty(n_rows + 1, dtype=torch.int64, device=dev)
             result = torch.empty(4, dtype=torch.int64, device=dev)
-            rc = self.lib.akshar_decode_batch(self._h, kind, form, ids.data_ptr(), 0 if ids.dtype == torch.int32 else 1, n_ids,
+            rc = self.lib.akshar_decode_batch(self._h, kind, form, ids.data_ptr(), u16, n_ids,
                                               splits.data_ptr(), n_rows, out.data_ptr(), cap, out_off.data_ptr(), result.data_ptr(),
                                               ws.data_ptr(), ws.numel(), self._stream())
             if rc != 0:
                 self._err(rc, 'akshar_decode_batch')
-            total, _, bits = self._finish(result, 'decode', True)
+            total, _, bits, _ = self._finish(result)
             if bits & C.ST_BAD_ID:
                 raise IndexError('piece id is out of range.')         # what SentencePiece's DecodeIds raises
             if bits & C.ST_OVERFLOW:
@@ -445,7 +439,6 @@ class Engine:
         and truncation takes True / 'longest_first', 'only_first', 'only_second', or False / 'do_not_truncate'.
         Raises ValueError where HF would misbehave (see the header) and for ids the encoder of this model did not produce.
         One read-back of the result block (N, longest window, status); nothing else synchronises."""
-        values, splits = (ids.values, ids.splits) if isinstance(ids, Ragged) else ids
         only = 0
         if pair_ids is not None:
             strategies = {'longest_first': 0, 'only_first': C.WIN_ONLY_FIRST, 'only_second': C.WIN_ONLY_SECOND}
@@ -470,46 +463,36 @@ class Engine:
             if pad_id is None:
                 raise ValueError('the model has no pad piece: pass pad_id')
         dev = self.device
-        values, splits = values.to(dev), splits.to(dev, torch.int64)
-        if values.dtype not in (torch.int32, torch.uint16, torch.int16):
-            values = values.to(torch.int32)
+        values, splits, u16 = self._ids_in(ids)
         if pair_ids is not None:
-            values_b, splits_b = (pair_ids.values, pair_ids.splits) if isinstance(pair_ids, Ragged) else pair_ids
-            values_b, splits_b = values_b.to(dev), splits_b.to(dev, torch.int64)
-            if values_b.dtype not in (torch.int32, torch.uint16, torch.int16):
-                values_b = values_b.to(torch.int32)
-            if (values.dtype == torch.int32) != (values_b.dtype == torch.int32):
-                values, values_b = _ids_int32(values), _ids_int32(values_b)
+            values_b, splits_b, u16_b = self._ids_in(pair_ids)
+            if u16 != u16_b:
+                values, values_b, u16 = _ids_int32(values), _ids_int32(values_b), 0
             if splits_b.numel() != splits.numel():
                 raise ValueError('ids and pair_ids must hold the same number of rows')
             if values_b.numel() >= 2 ** 31:
                 raise ValueError('windows_batch takes fewer than 2^31 ids per call')
         if values.numel() >= 2 ** 31:
             raise ValueError('windows_batch takes fewer than 2^31 ids per call')
-        u16 = 0 if values.dtype == torch.int32 else 1
         n_rows = splits.numel() - 1
         flags = ((C.WIN_TRUNCATE if truncation else 0) | (C.WIN_OVERFLOW if return_overflowing_tokens else 0) |
                  (C.WIN_TRUNC_LEFT if truncation_side == 'left' else 0) | (C.WIN_PAD_LEFT if padding_side == 'left' else 0) | only)
         ml = max_length if max_length is not None else 0
-        need = self.lib.akshar_windows_workspace_bytes(n_rows)
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = None
-            self._ws = torch.empty(need + (need >> 3), dtype=torch.uint8, device=dev)
+        ws = self._grow_ws(self.lib.akshar_windows_workspace_bytes(n_rows))
         wsplits = torch.empty(n_rows + 1, dtype=torch.int64, device=dev)
         result = torch.empty(4, dtype=torch.int64, device=dev)
         if pair_ids is None:
             rc = self.lib.akshar_windows_count(self._h, kind, values.data_ptr(), u16, splits.data_ptr(), n_rows, ml, stride, flags,
-                                               wsplits.data_ptr(), result.data_ptr(), self._ws.data_ptr(), self._ws.numel(),
-                                               self._stream())
+                                               wsplits.data_ptr(), result.data_ptr(), ws.data_ptr(), ws.numel(), self._stream())
         else:
             rc = self.lib.akshar_pair_windows_count(self._h, kind, values.data_ptr(), splits.data_ptr(), values_b.data_ptr(),
                                                     splits_b.data_ptr(), u16, n_rows, ml, stride, flags, wsplits.data_ptr(),
-                                                    result.data_ptr(), self._ws.data_ptr(), self._ws.numel(), self._stream())
+                                                    result.data_ptr(), ws.data_ptr(), ws.numel(), self._stream())
         if rc == C.E_ARG:
             raise ValueError(self.lib.akshar_last_error(self._h).decode())
         if rc != 0:
             self._err(rc, 'akshar_pair_windows_count' if pair_ids is not None else 'akshar_windows_count')
-        n, longest, bits, refused = (int(x) for x in result.cpu())
+        n, longest, bits, refused = self._finish(result)
         if bits & C.ST_TEMPLATE:
             raise ValueError('a row does not begin / end with the template ids of the model: not ids of its encoder')
         if bits & C.ST_PAIR_TRUNC:
@@ -565,10 +548,7 @@ class Engine:
         if isinstance(separator_id, bool) or not isinstance(separator_id, int) or not -2 ** 63 <= separator_id < 2 ** 63:
             raise ValueError('separator_id must be an int64')
         dev = self.device
-        values, splits = (ids.values, ids.splits) if isinstance(ids, Ragged) else ids
-        values, splits = values.to(dev), splits.to(dev, torch.int64)
-        if values.dtype not in (torch.int32, torch.uint16, torch.int16):
-            values = values.to(torch.int32)
+        values, splits, u16 = self._ids_in(ids)
         if splits.dim() != 1 or splits.numel() < 1:
             raise ValueError('splits must be an int64 vector of n_rows + 1 positions')
         if carry is None:
@@ -588,14 +568,9 @@ class Engine:
             n_carry = cs.numel() - 1
         if values.numel() + (cv.numel() if cv is not None else 0) >= 2 ** 31:
             raise ValueError('pack_batch takes a stream of fewer than 2^31 ids per call (cu_seq_lens and seq_idx are int32)')
-        u16 = 0 if values.dtype == torch.int32 else 1
         n_rows = splits.numel() - 1
         eos = -1 if eos_id is None else eos_id
-        need = self.lib.akshar_pack_workspace_bytes(n_rows + n_carry)
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = None
-            self._ws = torch.empty(need + (need >> 3), dtype=torch.uint8, device=dev)
-        ws = self._ws
+        ws = self._grow_ws(self.lib.akshar_pack_workspace_bytes(n_rows + n_carry))
         p = lambda t: t.data_ptr() if t is not None and t.numel() else None
         args = (values.data_ptr() if values.numel() else None, u16, splits.data_ptr(), n_rows, p(cv), p(cs) if n_carry else None,
                 n_carry, block_size, eos)
@@ -605,7 +580,7 @@ class Engine:
             raise ValueError(self.lib.akshar_last_error(self._h).decode())
         if rc != 0:
             self._err(rc, 'akshar_pack_count')
-        n, n_pieces, bits, longest, total, n_frags, _, _ = (int(x) for x in result.cpu())
+        n, n_pieces, bits, longest, total, n_frags, _, _ = self._finish(result)
         if bits & C.ST_PACK_LONG:
             raise ValueError('the stream of this call holds %d ids: pack_batch takes fewer than 2^31 per call (cu_seq_lens '
                              'and seq_idx are int32)' % total)
@@ -720,8 +695,7 @@ class Engine:
                 self._err(rc, 'akshar_normalize_segment_batch')
             if not check:
                 return TextBatch(out, out_off, 0, -1), {'cluster': cm, 'run': rm, 'tags': tg, 'result': result, 'words': W}
-            r = result.cpu()
-            bits, total = int(r[2]), int(r[3])
+            _, _, bits, total = self._finish(result)
             if bits & C.ST_PATHOLOGICAL:
                 # a bounded look-back gave up: the two stages one after the other, the first in its row-sequential mode
                 norm = self.normalize_batch(b, normalize_roman, clean_hinglish)
@@ -740,26 +714,16 @@ class Engine:
         copy out of chunk k - 2 overlap on three streams.  What crosses the link back is the normalized text, its row
         offsets and 4 bits per normalized byte of boundary masks.  The results live in buffers the engine reuses (valid
         until the next call)."""
-        import os
         import numpy as np
-        from . import shard
-        if chunk_bytes is None:
-            chunk_bytes = int(os.environ.get('AKSHAR_CHUNK_MB', '64')) << 20
-        dev = self.device
+        P = _HostPipeline(self, self.__dict__.setdefault('_pipe2_cache', {}), h_data, h_off, chunk_bytes, '64')
         n_rows = h_off.numel() - 1
-        off_np = h_off.numpy()
-        total_bytes = int(off_np[-1] - off_np[0])
-        ranges = shard.chunk_rows(off_np, chunk_bytes)
-        max_b = max(int(off_np[hi] - off_np[lo]) for lo, hi in ranges)
-        max_r = max(hi - lo for lo, hi in ranges)
         nflags = (C.NORM_ROMAN if normalize_roman else 0) | (C.NORM_CLEAN if clean_hinglish else 0)
         sflags = C.SEG_CLUSTERS | C.SEG_RUNS | (C.SEG_MATRAS if matras else 0)
-        ncap = max_b + (max_b >> 3) + 1024
-        W = (ncap + 32) // 32
-        ws = self._workspace(ncap, max_r)
-        pc = self.__dict__.setdefault('_pipe2_cache', {})
+        W = (P.ncap + 32) // 32
+        pc = P.cache
+        total_bytes = int(P.off[-1] - P.off[0])
         est_b = total_bytes + (total_bytes >> 4) + 4096
-        est_w = (est_b + 32) // 32 + len(ranges) + 8
+        est_w = (est_b + 32) // 32 + len(P.ranges) + 8
         # pinned result buffers are kept and only ever grow
         if pc.get('norm') is None or pc['norm'].numel() < est_b:
             pc['norm'] = torch.empty(est_b + (est_b >> 4), dtype=torch.uint8).pin_memory()
@@ -768,101 +732,44 @@ class Engine:
         if pc.get('masks') is None or pc['masks'].shape[1] < est_w:
             pc['masks'] = torch.empty((4, est_w + (est_w >> 4)), dtype=torch.int32).pin_memory()
         h_norm, h_noff, h_masks = pc['norm'], pc['off'][:n_rows + 1], pc['masks']
-        if 'streams' not in pc:
-            pc['streams'] = tuple(torch.cuda.Stream(device=dev) for _ in range(3))
-        s_in, s_comp, s_out = pc['streams']
-        NSETS = 3
-        key = (max_b, max_r)
-        sets = pc.get('sets') if pc.get('sets_key') == key else None
-        if sets is None:
-            sets = [{
-                'text': torch.empty(max(max_b, 1), dtype=torch.uint8, device=dev),
-                'off': torch.empty(max_r + 1, dtype=torch.int64, device=dev),
-                'norm': torch.empty(max(ncap, 1), dtype=torch.uint8, device=dev),
-                'norm_off': torch.empty(max_r + 1, dtype=torch.int64, device=dev),
-                'masks': torch.empty((4, W), dtype=torch.int32, device=dev),
-                'result': torch.empty(4, dtype=torch.int64, device=dev),
-                'ev_in': torch.cuda.Event(), 'ev_comp': torch.cuda.Event(), 'ev_out': torch.cuda.Event(),
-            } for _ in range(NSETS)]
-        pc['sets'], pc['sets_key'] = sets, key
-        cur = torch.cuda.current_stream(dev)
-        for st in (s_in, s_comp, s_out):
-            st.wait_stream(cur)
-        chunk_rows = np.array([lo for lo, _ in ranges] + [n_rows], dtype=np.int64)
-        chunk_b = np.zeros(len(ranges) + 1, dtype=np.int64)
-        chunk_w = np.zeros(len(ranges) + 1, dtype=np.int64)
+        chunk_b = np.zeros(len(P.ranges) + 1, dtype=np.int64)
+        chunk_w = np.zeros(len(P.ranges) + 1, dtype=np.int64)
         state = {'b': 0, 'w': 0, 'c': 0, 'r': 0}
 
-        def finish(k):
-            lo, hi = ranges[k]
-            S = sets[k % NSETS]
-            with torch.cuda.stream(s_out):
-                s_out.wait_event(S['ev_comp'])
-                r = S['result'].cpu()
-                bits, nb = int(r[2]), int(r[3])
-                norm, noff, masks = S['norm'], S['norm_off'], S['masks']
-                nc, nr = int(r[0]), int(r[1])
-                if bits:
-                    # this chunk again through the plain path (larger capacities / the row-sequential normalizer)
-                    self.redone_chunks = getattr(self, 'redone_chunks', 0) + 1
-                    # the plain path uses the engine's one workspace, which chunks k + 1 and k + 2 are still using on
-                    # s_comp: start it after them (its read-back then ends it before chunk k + 3)
-                    s_out.wait_stream(s_comp)
-                    b0, b1 = int(off_np[lo]), int(off_np[hi])
-                    nbatch, mk = self.normalize_segment_batch((h_data[b0:b1], h_off[lo:hi + 1] - b0), normalize_roman, clean_hinglish,
-                                                              True, matras, True)
-                    rr = mk['result'].cpu()
-                    nc, nr, nb = int(rr[0]), int(rr[1]), nbatch.end
-                    norm, noff = nbatch.data, nbatch.offsets
-                    masks = torch.stack([mk['cluster'], mk['run'], mk['tags'][0], mk['tags'][1]])
-                nw = (nb + 32) // 32
-                if state['b'] + nb > h_norm.numel() or state['w'] + nw > h_masks.shape[1]:
-                    raise BatchStatusError(C.ST_OVERFLOW, 'pipeline_host_pipelined: the normalized text grew beyond the pinned result buffers')
-                h_norm[state['b']:state['b'] + nb].copy_(norm[:nb], non_blocking=True)
-                h_noff[lo + 1:hi + 1].copy_(noff[1:hi - lo + 1] + state['b'], non_blocking=True)
-                for pl in range(4):              # plane by plane: contiguous copies (a strided 2-D copy would be staged)
-                    h_masks[pl, state['w']:state['w'] + nw].copy_(masks[pl, :nw], non_blocking=True)
-                S['ev_out'].record(s_out)
-                chunk_b[k], chunk_w[k] = state['b'], state['w']
-                state['b'] += nb
-                state['w'] += nw
-                state['c'] += nc
-                state['r'] += nr
+        def launch(S, b0, b1, nr, ws, stream):
+            m = S['masks']
+            rc = self.lib.akshar_normalize_segment_batch(
+                self._h, S['text'].data_ptr() - b0, S['off'].data_ptr(), nr, b0, b1, nflags, sflags, S['norm'].data_ptr(), P.ncap,
+                S['norm_off'].data_ptr(), m[0].data_ptr(), m[1].data_ptr(), m[2].data_ptr(), W, S['result'].data_ptr(),
+                ws.data_ptr(), ws.numel(), stream)
+            if rc != 0:
+                self._err(rc, 'akshar_normalize_segment_batch')
+
+        def redo(sub):
+            nbatch, mk = self.normalize_segment_batch(sub, normalize_roman, clean_hinglish, True, matras, True)
+            rr = mk['result'].cpu()
+            masks = torch.stack([mk['cluster'], mk['run'], mk['tags'][0], mk['tags'][1]])
+            return (int(rr[0]), int(rr[1]), 0, nbatch.end), {'norm': nbatch.data, 'norm_off': nbatch.offsets, 'masks': masks}
+
+        def copy_out(k, lo, hi, r, bufs):
+            nc, nr, _, nb = r
+            nw = (nb + 32) // 32
+            if state['b'] + nb > h_norm.numel() or state['w'] + nw > h_masks.shape[1]:
+                raise BatchStatusError(C.ST_OVERFLOW, 'pipeline_host_pipelined: the normalized text grew beyond the pinned result buffers')
+            h_norm[state['b']:state['b'] + nb].copy_(bufs['norm'][:nb], non_blocking=True)
+            h_noff[lo + 1:hi + 1].copy_(bufs['norm_off'][1:hi - lo + 1] + state['b'], non_blocking=True)
+            for pl in range(4):              # plane by plane: contiguous copies (a strided 2-D copy would be staged)
+                h_masks[pl, state['w']:state['w'] + nw].copy_(bufs['masks'][pl, :nw], non_blocking=True)
+            chunk_b[k], chunk_w[k] = state['b'], state['w']
+            state['b'] += nb
+            state['w'] += nw
+            state['c'] += nc
+            state['r'] += nr
 
         h_noff[0] = 0
-        try:
-            for k, (lo, hi) in enumerate(ranges):
-                S = sets[k % NSETS]
-                b0, b1 = int(off_np[lo]), int(off_np[hi])
-                nb, nr = b1 - b0, hi - lo
-                with torch.cuda.stream(s_in):
-                    if k >= NSETS:
-                        s_in.wait_event(S['ev_comp'])
-                    S['text'][:nb].copy_(h_data[b0:b1], non_blocking=True)
-                    S['off'][:nr + 1].copy_(h_off[lo:hi + 1], non_blocking=True)
-                    S['ev_in'].record(s_in)
-                with torch.cuda.stream(s_comp):
-                    s_comp.wait_event(S['ev_in'])
-                    if k >= NSETS:
-                        s_comp.wait_event(S['ev_out'])
-                    m = S['masks']
-                    rc = self.lib.akshar_normalize_segment_batch(
-                        self._h, S['text'].data_ptr() - b0, S['off'].data_ptr(), nr, b0, b1, nflags, sflags, S['norm'].data_ptr(), ncap,
-                        S['norm_off'].data_ptr(), m[0].data_ptr(), m[1].data_ptr(), m[2].data_ptr(), W, S['result'].data_ptr(),
-                        ws.data_ptr(), ws.numel(), ctypes.c_void_p(s_comp.cuda_stream))
-                    if rc != 0:
-                        self._err(rc, 'akshar_normalize_segment_batch')
-                    S['ev_comp'].record(s_comp)
-                if k >= 2:
-                    finish(k - 2)
-            for k in range(max(0, len(ranges) - 2), len(ranges)):
-                finish(k)
-        finally:
-            for st in (s_in, s_comp, s_out):
-                cur.wait_stream(st)
-            torch.cuda.synchronize(dev)
-        chunk_b[len(ranges)], chunk_w[len(ranges)] = state['b'], state['w']
-        return PipelineOut(h_norm[:state['b']], h_noff, h_masks[0], h_masks[1], h_masks[2], h_masks[3], chunk_rows, chunk_b, chunk_w,
+        P.run((), lambda: {'masks': torch.empty((4, W), dtype=torch.int32, device=self.device)}, launch, redo, copy_out)
+        chunk_b[-1], chunk_w[-1] = state['b'], state['w']
+        return PipelineOut(h_norm[:state['b']], h_noff, h_masks[0], h_masks[1], h_masks[2], h_masks[3], P.chunk_rows, chunk_b, chunk_w,
                            state['c'], state['r'])
 
     # ------------------------------------------------------------------ K1b
@@ -879,7 +786,7 @@ class Engine:
                                              ws.numel(), self._stream())
         if rc != 0:
             self._err(rc, 'akshar_signature_batch')
-        total, _, bits = self._finish(result, 'signature', True)
+        total, _, bits, _ = self._finish(result)
         if bits:
             raise BatchStatusError(bits, 'signature_batch')
         return TextBatch(out, out_off, 0, total)
@@ -937,24 +844,34 @@ class Engine:
                 self._err(rc, what)
             if not check:
                 return Ragged(ids, splits), result
-            total, _, bits = self._finish(result, what, True)
-            if bits & C.ST_PATHOLOGICAL and mode == C.MODE_TILES:
-                mode = C.MODE_ROWS
-                continue
-            if bits & C.ST_WORD and word_extra < 64:
-                # a batch full of very long words ran out of the long-word pool: half of the workspace beyond the library's
-                # minimum goes to that pool (include/akshar_b200.h), so grow the workspace and call again
-                word_extra = 16 if word_extra == 0 else 64
-                ws = self._workspace(b.n_bytes, b.n_rows, extra=word_extra * b.n_bytes + (4 << 20))
-                continue
-            if bits & C.ST_OVERFLOW:
-                cap = max(cap, total)
-                ws = self._workspace(b.n_bytes, b.n_rows, extra=max(ws.numel() - self.lib.akshar_workspace_bytes(b.n_bytes, b.n_rows), self._slot_extra(b.n_bytes)))
-                continue
-            if bits:
-                raise BatchStatusError(bits, what)
-            return Ragged(ids[:total], splits)
-        raise BatchStatusError(bits, what + ' (retries exhausted)')
+            r = self._finish(result)
+            if not r[2]:
+                return Ragged(ids[:r[0]], splits)
+            mode, word_extra, ws, cap, _ = self._encoder_retry(r, what, mode, word_extra, ws, cap, b.n_bytes, b.n_bytes, b.n_rows)
+        raise BatchStatusError(r[2], what + ' (retries exhausted)')
+
+    def _encoder_retry(self, r, what, mode, word_extra, ws, cap, ncap, n_bytes, n_rows):
+        """what an encoder call changes before it tries again after the result block `r` raised status bits -> (mode,
+        word_extra, ws, cap, ncap); BatchStatusError when nothing helps.  cap: the id capacity; ncap: the text bytes the
+        workspace is sized for, which grows to the normalized bytes r[1] of akshar_tokenizer_encode_batch (the encoders of
+        normalized rows leave r[1] at 0); n_bytes: the bytes of the batch; n_rows: its rows"""
+        total, nbytes, bits, slots = r
+        if bits & C.ST_PATHOLOGICAL and mode == C.MODE_TILES:
+            return C.MODE_ROWS, word_extra, ws, cap, ncap
+        if bits & C.ST_WORD and word_extra < 64:
+            # a batch full of very long words ran out of the long-word pool: half of the workspace beyond the library's
+            # minimum goes to that pool (include/akshar_b200.h), so grow the workspace and call again
+            word_extra = 16 if word_extra == 0 else 64
+            return mode, word_extra, self._workspace(ncap, n_rows, extra=word_extra * n_bytes + (4 << 20)), cap, ncap
+        if bits & C.ST_OVERFLOW:
+            # totals are exact even when a capacity was too small
+            cap = max(cap, total)
+            if nbytes > ncap:
+                ncap = nbytes
+                cap = max(cap, (ncap >> 1) + 2 * n_rows + 1024)
+            extra = max(ws.numel() - self.lib.akshar_workspace_bytes(ncap, n_rows), self._slot_extra(ncap, slots))
+            return mode, word_extra, self._workspace(ncap, n_rows, extra=extra), cap, ncap
+        raise BatchStatusError(bits, what)
 
     def encode_bpe_batch(self, batch, mode=C.MODE_TILES, capacity=None, check=True):
         """Tokenizer.encode(norm).ids over ALREADY NORMALIZED rows (reference tokenizer.py:193) -> Ragged int32 ids"""
@@ -990,26 +907,12 @@ class Engine:
                 self._err(rc, 'akshar_tokenizer_encode_batch')
             if not check:
                 return Ragged(ids, splits), TextBatch(norm, norm_off, 0, -1), result
-            total, nbytes, bits = self._finish(result, 'tokenizer_encode', True)
-            if bits & C.ST_PATHOLOGICAL and mode == C.MODE_TILES:
-                mode = C.MODE_ROWS
-                continue
-            if bits & C.ST_WORD and word_extra < 64:
-                word_extra = 16 if word_extra == 0 else 64         # long-word pool: see _encode
-                ws = self._workspace(ncap, b.n_rows, extra=word_extra * b.n_bytes + (4 << 20))
-                continue
-            if bits & C.ST_OVERFLOW:
-                # totals are exact even when a capacity was too small
-                cap = max(cap, total)
-                if nbytes > ncap:
-                    ncap = nbytes
-                    cap = max(cap, (ncap >> 1) + 2 * b.n_rows + 1024)
-                ws = self._workspace(ncap, b.n_rows, extra=max(ws.numel() - self.lib.akshar_workspace_bytes(ncap, b.n_rows), self._slot_extra(ncap)))
-                continue
-            if bits:
-                raise BatchStatusError(bits, 'tokenizer_encode_batch')
-            return Ragged(ids[:total], splits), TextBatch(norm, norm_off, 0, nbytes)
-        raise BatchStatusError(bits, 'tokenizer_encode_batch (retries exhausted)')
+            r = self._finish(result)
+            if not r[2]:
+                return Ragged(ids[:r[0]], splits), TextBatch(norm, norm_off, 0, r[1])
+            mode, word_extra, ws, cap, ncap = self._encoder_retry(r, 'tokenizer_encode_batch', mode, word_extra, ws, cap, ncap,
+                                                                  b.n_bytes, b.n_rows)
+        raise BatchStatusError(r[2], 'tokenizer_encode_batch (retries exhausted)')
 
 
     # ------------------------------------------------------------------ host -> ids, pipelined
@@ -1028,31 +931,22 @@ class Engine:
         valid until the next call of this method on the same engine (pinning fresh memory for every call would cost more
         than the call).  A caller that needs them longer passes its own pinned tensors; a tensor that is too small is an
         error, it is never swapped silently."""
-        import os
         import numpy as np
-        from . import shard
-        if chunk_bytes is None:
-            # 64 MiB keeps both copy engines busy for BPE; the Unigram path has a latency floor per call (its exact-Viterbi
-            # check walks whole rows), which 128 MiB chunks amortize (measured: 32 -> 40 GB/s end to end)
-            chunk_bytes = int(os.environ.get('AKSHAR_CHUNK_MB', '64' if kind == 0 else '128')) << 20
-        dev = self.device
         n_rows = h_off.numel() - 1
-        off_np = h_off.numpy()
-        total_bytes = int(off_np[-1] - off_np[0])
-        ranges = shard.chunk_rows(off_np, chunk_bytes)
-        max_b = max(int(off_np[hi] - off_np[lo]) for lo, hi in ranges)
-        max_r = max(hi - lo for lo, hi in ranges)
         flags = (C.NORM_ROMAN if normalize_roman else 0) | (C.NORM_CLEAN if clean_hinglish else 0)
         if compact and self.lib.akshar_vocab_size(self._h, kind) > 65536:
             raise ValueError('compact ids need a vocabulary of at most 65536 entries')
         out_flags = (C.OUT_IDS_U16 | C.OUT_SPLITS_I32) if compact else 0
         id_dtype = torch.int16 if compact else torch.int32          # (uint16 bit patterns; torch copies them as they are)
         sp_dtype = torch.int32 if compact else torch.int64
-        ncap = max_b + (max_b >> 3) + 1024
-        cap = (max_b >> 1) + 2 * max_r + 1024
-        ws = self._workspace(ncap, max_r)
-        # pinned result buffers, device double buffers and streams are kept by the engine: repeated calls allocate nothing
-        pc = self.__dict__.setdefault('_pipe_cache', {})
+        # 64 MiB keeps both copy engines busy for BPE; the Unigram path has a latency floor per call (its exact-Viterbi
+        # check walks whole rows), which 128 MiB chunks amortize (measured: 32 -> 40 GB/s end to end)
+        P = _HostPipeline(self, self.__dict__.setdefault('_pipe_cache', {}), h_data, h_off, chunk_bytes,
+                          '64' if kind == 0 else '128')
+        cap = (P.max_b >> 1) + 2 * P.max_r + 1024
+        # pinned result buffers, device buffer sets and streams are kept by the engine: repeated calls allocate nothing
+        pc = P.cache
+        total_bytes = int(P.off[-1] - P.off[0])
         est = (total_bytes >> 1) + 2 * n_rows + 1024
         key_sp, key_id = ('splits', sp_dtype), ('ids', id_dtype)
         if out_splits is None:
@@ -1068,33 +962,105 @@ class Engine:
             out_ids = pc[key_id]
         elif out_ids.dtype != id_dtype:
             raise ValueError('out_ids must be %s' % id_dtype)
+        chunk_ids = np.zeros(len(P.ranges) + 1, dtype=np.int64)
+        state = {'tok': 0, 'ids': out_ids}
+
+        def launch(S, b0, b1, nr, ws, stream):
+            rc = self.lib.akshar_tokenizer_encode_batch_ex(
+                self._h, S['text'].data_ptr() - b0, S['off'].data_ptr(), nr, b0, b1, flags, kind, C.MODE_TILES,
+                S['norm'].data_ptr(), P.ncap, S['norm_off'].data_ptr(), S['ids'].data_ptr(), cap, S['splits'].data_ptr(),
+                out_flags, S['result'].data_ptr(), ws.data_ptr(), ws.numel(), stream)
+            if rc != 0:
+                self._err(rc, 'akshar_tokenizer_encode_batch_ex')
+
+        def redo(sub):
+            ids, _ = self.tokenizer_encode_batch(sub, kind, normalize_roman, clean_hinglish)
+            v, sp = ids.values, ids.splits
+            if compact:
+                v, sp = v.to(torch.int16), sp.to(torch.int32)
+            return (v.numel(), 0, 0, 0), {'ids': v, 'splits': sp}
+
+        def copy_out(k, lo, hi, r, bufs):
+            n, tok, dst = r[0], state['tok'], state['ids']
+            if tok + n > dst.numel():
+                if own_ids:
+                    raise ValueError('out_ids is too small: %d ids so far, %d more in this chunk' % (tok, n))
+                grown = torch.empty(max(2 * dst.numel(), tok + n), dtype=id_dtype).pin_memory()
+                torch.cuda.synchronize(self.device)
+                grown[:tok].copy_(dst[:tok])
+                dst = state['ids'] = pc[key_id] = grown
+            dst[tok:tok + n].copy_(bufs['ids'][:n], non_blocking=True)
+            sp = bufs['splits'][1:hi - lo + 1]
+            if not compact and tok:
+                sp = sp + tok
+            out_splits[lo + 1:hi + 1].copy_(sp, non_blocking=True)
+            chunk_ids[k] = tok
+            state['tok'] = tok + n
+
+        out_splits[0] = 0
+        P.run((compact,), lambda: {'ids': torch.empty(max(cap, 1), dtype=id_dtype, device=self.device),
+                                   'splits': torch.empty(P.max_r + 1, dtype=sp_dtype, device=self.device)},
+              launch, redo, copy_out)
+        out_ids, tok = state['ids'], state['tok']
+        chunk_ids[-1] = tok
+        if compact:
+            return CompactIds(out_ids[:tok], out_splits[:n_rows + 1], P.chunk_rows, chunk_ids)
+        return out_ids[:tok], out_splits[:n_rows + 1]
+
+
+class _HostPipeline:
+    """A batch in pinned host memory through the device in chunks of rows: the rows are cut into ranges of about
+    chunk_bytes (AKSHAR_CHUNK_MB MiB by default) that keep their absolute offsets, and the copy in of chunk k + 1, the
+    kernels of chunk k and the copy out of chunk k - 2 overlap on three streams.  A path sizes its buffers from the cut
+    (`ranges`; `max_b` bytes and `max_r` rows of the largest chunk, `ncap` bytes of its normalized text), then `run`s it
+    with its own ABI call, copy-out and plain-path redo of one chunk.  `cache` is a dict of the path's own on the engine:
+    the streams and the device buffer sets stay there between calls."""
+
+    NSETS = 3        # input / compute / output of three consecutive chunks in flight; the host trails two chunks behind
+
+    def __init__(self, eng, cache, h_data, h_off, chunk_bytes, default_mb):
+        import os
+        import numpy as np
+        from . import shard
+        if chunk_bytes is None:
+            chunk_bytes = int(os.environ.get('AKSHAR_CHUNK_MB', default_mb)) << 20
+        self.trace = [] if os.environ.get('AKSHAR_PIPE_TRACE') else None
+        self.eng, self.cache, self.h_data, self.h_off = eng, cache, h_data, h_off
+        self.off = off = h_off.numpy()
+        self.ranges = shard.chunk_rows(off, chunk_bytes)
+        self.max_b = max(int(off[hi] - off[lo]) for lo, hi in self.ranges)
+        self.max_r = max(hi - lo for lo, hi in self.ranges)
+        self.ncap = self.max_b + (self.max_b >> 3) + 1024
+        # the workspace of every chunk of the call: a redo may replace the engine's, this one lives until the call ends
+        self.ws = eng._workspace(self.ncap, self.max_r)
+        self.chunk_rows = np.array([lo for lo, _ in self.ranges] + [h_off.numel() - 1], dtype=np.int64)
+
+    def run(self, key, set_bufs, launch, redo, copy_out):
+        """key: what besides the chunk shape selects the cached buffer sets; set_bufs() -> the path's own device buffers
+        of one set; launch(S, b0, b1, rows, ws, stream): the ABI call on the chunk in set S (bytes b0 .. b1 of the batch);
+        redo(sub) -> (result, buffers): the chunk's rows, a host (data, offsets) pair, through the plain path;
+        copy_out(k, lo, hi, result, buffers): chunk k (rows lo .. hi - 1) to the host, from its set and its 4-word
+        result block or from what redo returned.  redo and copy_out run on the copy-out stream."""
+        eng, pc, dev, NSETS, trace = self.eng, self.cache, self.eng.device, self.NSETS, self.trace
+        ranges, off, h_data, h_off = self.ranges, self.off, self.h_data, self.h_off
         if 'streams' not in pc:
             pc['streams'] = tuple(torch.cuda.Stream(device=dev) for _ in range(3))
         s_in, s_comp, s_out = pc['streams']
-        NSETS = 3        # input / compute / output of three consecutive chunks in flight; the host trails two chunks behind
-        key = (max_b, max_r, NSETS, compact)
+        key = (self.max_b, self.max_r) + key
         sets = pc.get('sets') if pc.get('sets_key') == key else None
         if sets is None:
-            sets = []
-            for _ in range(NSETS):
-                sets.append({
-                    'text': torch.empty(max(max_b, 1), dtype=torch.uint8, device=dev),
-                    'off': torch.empty(max_r + 1, dtype=torch.int64, device=dev),
-                    'norm': torch.empty(max(ncap, 1), dtype=torch.uint8, device=dev),
-                    'norm_off': torch.empty(max_r + 1, dtype=torch.int64, device=dev),
-                    'ids': torch.empty(max(cap, 1), dtype=id_dtype, device=dev),
-                    'splits': torch.empty(max_r + 1, dtype=sp_dtype, device=dev),
-                    'result': torch.empty(4, dtype=torch.int64, device=dev),
-                    'ev_in': torch.cuda.Event(), 'ev_comp': torch.cuda.Event(), 'ev_out': torch.cuda.Event(),
-                })
+            sets = [{'text': torch.empty(max(self.max_b, 1), dtype=torch.uint8, device=dev),
+                     'off': torch.empty(self.max_r + 1, dtype=torch.int64, device=dev),
+                     'norm': torch.empty(max(self.ncap, 1), dtype=torch.uint8, device=dev),
+                     'norm_off': torch.empty(self.max_r + 1, dtype=torch.int64, device=dev),
+                     **set_bufs(),
+                     'result': torch.empty(4, dtype=torch.int64, device=dev),
+                     'ev_in': torch.cuda.Event(), 'ev_comp': torch.cuda.Event(), 'ev_out': torch.cuda.Event()}
+                    for _ in range(NSETS)]
         pc['sets'], pc['sets_key'] = sets, key
         cur = torch.cuda.current_stream(dev)
         for st in (s_in, s_comp, s_out):
             st.wait_stream(cur)
-        state = {'tok': 0}
-        chunk_rows = np.array([lo for lo, _ in ranges] + [n_rows], dtype=np.int64)
-        chunk_ids = np.zeros(len(ranges) + 1, dtype=np.int64)
-        trace = [] if os.environ.get('AKSHAR_PIPE_TRACE') else None
         if trace is not None:
             t0ev = torch.cuda.Event(enable_timing=True)
             t0ev.record(cur)
@@ -1105,81 +1071,45 @@ class Engine:
                 e.record(stream)
                 trace.append((what, k, e))
 
-        def redo_chunk(k):
-            """a chunk whose fast call raised a status: the same rows through the plain path (which retries with larger
-            capacities / the row-by-row mode) -- only this chunk, the others keep their results"""
-            lo, hi = ranges[k]
-            b0, b1 = int(off_np[lo]), int(off_np[hi])
-            sub = (h_data[b0:b1], (h_off[lo:hi + 1] - b0))
-            with torch.cuda.stream(s_out):
-                ids, _ = self.tokenizer_encode_batch(sub, kind, normalize_roman, clean_hinglish)
-                v = ids.values
-                sp = ids.splits
-                if compact:
-                    v = v.to(torch.int16)
-                    sp = sp.to(torch.int32)
-                return v, sp, int(v.numel())
-
         def finish(k):
             lo, hi = ranges[k]
             S = sets[k % NSETS]
             with torch.cuda.stream(s_out):
                 s_out.wait_event(S['ev_comp'])
-                r = S['result'].cpu()          # waits for chunk k's kernels only; later chunks are already enqueued
-                n, bits = int(r[0]), int(r[2])
-                d_ids, d_sp = S['ids'], S['splits']
-                if bits:
-                    self.redone_chunks = getattr(self, 'redone_chunks', 0) + 1
+                r = eng._finish(S['result'])       # waits for chunk k's kernels only; later chunks are already enqueued
+                bufs = S
+                if r[2]:
+                    # this chunk alone again through the plain path (larger capacities / the row-sequential modes)
+                    eng.redone_chunks = getattr(eng, 'redone_chunks', 0) + 1
                     # the plain path uses the engine's one workspace and the model's word cache, which chunks k + 1 and
                     # k + 2 are still using on s_comp: start it after them (its read-back then ends it before chunk k + 3)
                     s_out.wait_stream(s_comp)
-                    d_ids, d_sp, n = redo_chunk(k)
-                if state['tok'] + n > out_ids.numel():
-                    if own_ids:
-                        raise ValueError('out_ids is too small: %d ids so far, %d more in this chunk' % (state['tok'], n))
-                    grown = torch.empty(max(2 * out_ids.numel(), state['tok'] + n), dtype=id_dtype).pin_memory()
-                    torch.cuda.synchronize(dev)
-                    grown[:state['tok']].copy_(out_ids[:state['tok']])
-                    pc[key_id] = grown
-                    state['out_ids'] = grown
-                dst = state.get('out_ids', out_ids)
+                    b0, b1 = int(off[lo]), int(off[hi])
+                    r, bufs = redo((h_data[b0:b1], h_off[lo:hi + 1] - b0))
                 mark(s_out, 'd2h_begin', k)
-                dst[state['tok']:state['tok'] + n].copy_(d_ids[:n], non_blocking=True)
-                sp = d_sp[1:hi - lo + 1]
-                if not compact and state['tok']:
-                    sp = sp + state['tok']
-                out_splits[lo + 1:hi + 1].copy_(sp, non_blocking=True)
+                copy_out(k, lo, hi, r, bufs)
                 S['ev_out'].record(s_out)
                 mark(s_out, 'd2h_end', k)
-                chunk_ids[k] = state['tok']
-                state['tok'] += n
 
-        out_splits[0] = 0
         try:
             for k, (lo, hi) in enumerate(ranges):
                 S = sets[k % NSETS]
-                b0, b1 = int(off_np[lo]), int(off_np[hi])
-                nb, nr = b1 - b0, hi - lo
+                b0, b1 = int(off[lo]), int(off[hi])
                 with torch.cuda.stream(s_in):
                     if k >= NSETS:
                         s_in.wait_event(S['ev_comp'])      # the kernels that read this input buffer have finished
                     # the rows keep their ABSOLUTE offsets (the C ABI takes text_begin / text_end): no per-chunk rebasing on
                     # the host, the offsets go to the device straight from the caller's (pinned) array
                     mark(s_in, 'h2d_begin', k)
-                    S['text'][:nb].copy_(h_data[b0:b1], non_blocking=True)
-                    S['off'][:nr + 1].copy_(h_off[lo:hi + 1], non_blocking=True)
+                    S['text'][:b1 - b0].copy_(h_data[b0:b1], non_blocking=True)
+                    S['off'][:hi - lo + 1].copy_(h_off[lo:hi + 1], non_blocking=True)
                     S['ev_in'].record(s_in)
                     mark(s_in, 'h2d_end', k)
                 with torch.cuda.stream(s_comp):
                     s_comp.wait_event(S['ev_in'])
                     if k >= NSETS:
-                        s_comp.wait_event(S['ev_out'])     # chunk k-NSETS's results left this set's output buffers
-                    rc = self.lib.akshar_tokenizer_encode_batch_ex(
-                        self._h, S['text'].data_ptr() - b0, S['off'].data_ptr(), nr, b0, b1, flags, kind, C.MODE_TILES,
-                        S['norm'].data_ptr(), ncap, S['norm_off'].data_ptr(), S['ids'].data_ptr(), cap, S['splits'].data_ptr(),
-                        out_flags, S['result'].data_ptr(), ws.data_ptr(), ws.numel(), ctypes.c_void_p(s_comp.cuda_stream))
-                    if rc != 0:
-                        self._err(rc, 'akshar_tokenizer_encode_batch_ex')
+                        s_comp.wait_event(S['ev_out'])     # chunk k - NSETS's results left this set's output buffers
+                    launch(S, b0, b1, hi - lo, self.ws, ctypes.c_void_p(s_comp.cuda_stream))
                     S['ev_comp'].record(s_comp)
                     mark(s_comp, 'comp_end', k)
                 if k >= 2:
@@ -1192,11 +1122,6 @@ class Engine:
             torch.cuda.synchronize(dev)
         if trace:
             print('pipe trace (ms): ' + ' '.join('%s%d=%.2f' % (w, k, t0ev.elapsed_time(e)) for w, k, e in trace))
-        out_ids = state.get('out_ids', out_ids)
-        chunk_ids[len(ranges)] = state['tok']
-        if compact:
-            return CompactIds(out_ids[:state['tok']], out_splits[:n_rows + 1], chunk_rows, chunk_ids)
-        return out_ids[:state['tok']], out_splits[:n_rows + 1]
 
 
 class PipelineOut:

@@ -17,39 +17,8 @@ _STAGE_FLAGS = {
 
 
 def _run_flags(batch, flags, as_device=False, device=0):
-    eng = engine(device)
-    b = eng.put(batch)
-    lib = eng.lib
-    import ctypes
-    import torch
-    ws = eng._workspace(b.n_bytes, b.n_rows)
-    cap = b.n_bytes + (b.n_bytes >> 3) + 1024
-    mode = C.MODE_TILES
-    for _ in range(eng.MAX_TRIES):
-        out = torch.empty(max(cap, 1), dtype=torch.uint8, device=eng.device)
-        out_off = torch.empty(b.n_rows + 1, dtype=torch.int64, device=eng.device)
-        result = torch.empty(4, dtype=torch.int64, device=eng.device)
-        rc = lib.akshar_normalize_batch(eng._h, b.data.data_ptr(), b.offsets.data_ptr(), b.n_rows, b.begin, b.end, flags, mode,
-                                        out.data_ptr(), cap, out_off.data_ptr(), result.data_ptr(), ws.data_ptr(), ws.numel(),
-                                        eng._stream())
-        if rc != 0:
-            eng._err(rc, 'akshar_normalize_batch')
-        r = result.cpu()
-        total, bits = int(r[0]), int(r[2])
-        if bits & C.ST_PATHOLOGICAL and mode == C.MODE_TILES:
-            mode = C.MODE_ROWS
-            continue
-        if bits & C.ST_OVERFLOW:
-            cap = total
-            continue
-        if bits:
-            from .batch import BatchStatusError
-            raise BatchStatusError(bits, 'normalize')
-        from .batch import TextBatch
-        tb = TextBatch(out, out_off, 0, total)
-        return tb if as_device else tb.to_strings()
-    from .batch import BatchStatusError
-    raise BatchStatusError(bits, 'normalize (retries exhausted)')
+    tb = engine(device)._normalize(batch, flags)
+    return tb if as_device else tb.to_strings()
 
 
 def _norm_flags(normalize_roman, clean_hinglish):
