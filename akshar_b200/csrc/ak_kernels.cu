@@ -10,6 +10,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <exception>
 #include <new>
 #include <string>
@@ -100,6 +101,38 @@ struct AkDeviceGuard {
         }                                                                                          \
     } while (0)
 
+// sets the text akshar_last_error returns and passes the status code on
+static int ak_fail(akshar_ctx* ctx, int code, std::string msg) {
+    ctx->err = std::move(msg);
+    return code;
+}
+
+static int ak_ws_short(akshar_ctx* ctx, size_t need) {
+    return ak_fail(ctx, AKSHAR_E_WORKSPACE, "workspace too small: need " + std::to_string(need) + " bytes");
+}
+
+// calls f with a value of the caller's id type: uint16_t when ids_u16, int32_t otherwise
+template <class F>
+static int ak_with_ids(int ids_u16, F f) {
+    return ids_u16 ? f(uint16_t()) : f(int32_t());
+}
+
+static inline size_t ak_align(size_t x) { return (x + 255) & ~(size_t)255; }
+// the tile states of one ak_scan_counts_kernel over at most n entries
+static inline size_t ak_scan_state_bytes(size_t n) { return ak_align((n / AKS_TILE + 2) * 8); }
+
+// Bump allocator of one workspace layout: every region starts 256-byte aligned.  With a null base it only adds up the
+// sizes, so one function both sizes a workspace (akshar_*_workspace_bytes, ak_ws_layout) and carves it (the launcher).
+struct AkCarve {
+    char* base;
+    size_t at;
+    template <class T>
+    void take(T*& p, size_t bytes) {
+        p = base ? (T*)(base + at) : nullptr;
+        at += ak_align(bytes);
+    }
+};
+
 template <class V>
 static int ak_upload(akshar_ctx* ctx, std::vector<void*>& owner, const V* src, size_t n, const V** dst) {
     void* d = nullptr;
@@ -138,10 +171,8 @@ int akshar_ctx_create(int device, akshar_ctx** out) {
     AK_CUDA(ctx, cudaSetDevice(device));
     cudaDeviceProp prop;
     AK_CUDA(ctx, cudaGetDeviceProperties(&prop, device));
-    if (prop.major < 10) {
-        ctx->err = "akshar_b200 is built for sm_100a (B200); device is sm_" + std::to_string(prop.major * 10 + prop.minor);
-        return AKSHAR_E_CUDA;
-    }
+    if (prop.major < 10)
+        return ak_fail(ctx, AKSHAR_E_CUDA, "akshar_b200 is built for sm_100a (B200); device is sm_" + std::to_string(prop.major * 10 + prop.minor));
     ctx->sm_count = prop.multiProcessorCount;
     int rc;
 #define UP(field, arr, n, type) \
@@ -251,12 +282,29 @@ int akshar_timing_read(akshar_ctx* ctx, int timer, float* ms) {
 
 int64_t akshar_launch_count(akshar_ctx* ctx) { return ctx ? ctx->launches : 0; }
 
-// workspace layout (all regions 256-byte aligned):
-//   [0, 256)            control block: tickets[8] (int), changed flag, pool cursor
-//   state regions       4 x n_tiles x 8 bytes (two counters x two passes)
-//   scratch             max(unigram back-pointers 4 (n_bytes + 2 n_rows + 2), signature code points 4 n_bytes,
-//                           BPE: NFC'd text n_bytes + n_bytes / 8 + 1024, its row offsets 8 (n_rows + 1), long-word pool)
-static inline size_t ak_align(size_t x) { return (x + 255) & ~(size_t)255; }
+// The first 256 bytes of every workspace, zeroed by each call before its first kernel.  A ticket hands out tile numbers
+// in the order the CTAs ask, so no two stages of one call may share one: the second would start at the first one's last
+// tile and skip the tiles before it.  The fused calls run the normalize stage (ticket or scan_b, n_slow) and then the
+// segment mask kernel (no control word) or an encoder (uni_rows, or scan_a, seg_scan and the event-stream words).
+struct AkControl {
+    int ticket;                      // tile ticket (AkBatch::ticket) of the walker kernels: generic normalize, generic
+                                     // segment, signatures; the scan ticket of decode, merge, lines, windows, pairs, pack
+    int uni_rows;                    // Unigram row kernel
+    int seg_scan;                    // event-stream Unigram: segmented scan
+    int scan_a;                      // scans: segment offsets' clusters, word tokenizer, event-stream encoders' ids
+    int scan_b;                      // scans: segment offsets' runs, fast normalize's output bytes
+    unsigned int n_slow;             // fast normalize: entries of the slow-lane work list
+    unsigned int any_flag;           // event-stream encoders: some row goes to the row-fix kernel
+    long long n_wt;                  // event-stream encoders: warp tiles the words kernel found (the scans' count)
+    unsigned long long longpool_used;  // event-stream encoders: long-word pool cursor
+    unsigned long long pool_used;    // event-stream encoders: id / Viterbi scratch pool cursor
+    unsigned long long pair_windows; // pair windows count: the windows of all pairs,
+    unsigned int pair_done;          // the blocks that have added theirs,
+    long long pair_n_scan;           // and the entries the scan takes (0 when the total does not fit its 32-bit tile sums)
+    int64_t pack_pieces;             // pack count: the scan's total
+};
+static_assert(sizeof(AkControl) <= 256, "the control block is the first 256 bytes of a workspace");
+
 static inline int64_t ak_tiles_of(int64_t n_bytes, int64_t n_rows) {
     int64_t a = (n_bytes + n_bytes / 8 + 1024 + 32 + AKF_TILE - 1) / AKF_TILE;     // fast-kernel tiles; covers the NFC'd copy too
     int64_t b = (n_rows + AK_ROWS_BLOCK - 1) / AK_ROWS_BLOCK;
@@ -280,7 +328,7 @@ static AkTokWs ak_tok_ws(int64_t n_bytes, int64_t n_rows) {
     W.wt_base = at;    at += ak_align((size_t)W.n_wt * 8);
     W.wt_seg = at;     at += ak_align((size_t)W.n_wt * 8);
     W.wt_segx = at;    at += ak_align((size_t)W.n_wt * 4);
-    W.scan_state = at; at += 2 * ak_align(((size_t)W.n_wt / AKS_TILE + 2) * 8);
+    W.scan_state = at; at += 2 * ak_scan_state_bytes((size_t)W.n_wt);
     W.row_flag = at;   at += ak_align((size_t)n_rows + 1);
     W.row_ev = at;     at += ak_align(((size_t)n_rows + 2) * 4);
     W.row_fix = at;    at += ak_align(((size_t)n_rows + 1) * 8);
@@ -294,8 +342,56 @@ static AkTokWs ak_tok_ws(int64_t n_bytes, int64_t n_rows) {
     return W;
 }
 
+// Scratch layouts of the text stages.  Each returns its size and, given a base, carves it; the launcher passes the tiles
+// it really has, ak_ws_layout the most the text can have.
+// fast normalize: per-lane info words, warp-tile totals and bases, the slow-lane work list
+static size_t ak_nf_ws(size_t n_tiles, char* base, AkNfWork& W) {
+    AkCarve c{base, 0};
+    c.take(W.info, n_tiles * AK_BLOCK * 4);
+    c.take(W.tile_total, n_tiles * AKF_WARPS * 4);
+    c.take(W.tile_base, (n_tiles * AKF_WARPS + 1) * 8);
+    const size_t slow_cap = n_tiles * AK_BLOCK / 16 + 1024;
+    W.slow_cap = (unsigned int)slow_cap;
+    c.take(W.slow, slow_cap * sizeof(AkSlowEntry));
+    return c.at;
+}
+// segment offsets: warp-tile row table, cluster and run counts and their bases per warp tile
+struct AkSegWs {
+    int64_t* wrow;
+    int32_t *c_count, *r_count;
+    int64_t *c_base, *r_base;
+};
+static size_t ak_seg_ws(size_t n_wt, char* base, AkSegWs& W) {
+    AkCarve c{base, 0};
+    c.take(W.wrow, (n_wt * 2 + 3) * 8);
+    c.take(W.c_count, n_wt * 4);
+    c.take(W.r_count, n_wt * 4);
+    c.take(W.c_base, n_wt * 8);
+    c.take(W.r_base, n_wt * 8);
+    return c.at;
+}
+// segment masks: the warp-tile row table
+static size_t ak_seg_mask_ws(size_t n_wt, char* base, int64_t*& wrow) {
+    AkCarve c{base, 0};
+    c.take(wrow, (n_wt * 2 + 3) * 8);
+    return c.at;
+}
+// word tokenizers: warp-tile row table, word counts and their bases per warp tile
+struct AkWtWs {
+    int64_t* wrow;
+    int32_t* count;
+    int64_t* base;
+};
+static size_t ak_wt_ws(size_t n_wt, char* base, AkWtWs& W) {
+    AkCarve c{base, 0};
+    c.take(W.wrow, (n_wt * 2 + 3) * 8);
+    c.take(W.count, n_wt * 4);
+    c.take(W.base, n_wt * 8);
+    return c.at;
+}
+
 struct AkWsLayout {
-    size_t control, state, tile_row, scratch, total;
+    size_t state, tile_row, scratch, total;
 };
 // [0, 256) control block, then the zeroed tile-state area (look-back states of the walker kernels, scan states), the
 // tile -> row table of the normalize kernels, and a scratch region shared by whatever stage runs: its size is the largest
@@ -303,24 +399,19 @@ struct AkWsLayout {
 static AkWsLayout ak_ws_layout(int64_t n_bytes, int64_t n_rows) {
     AkWsLayout L;
     size_t tiles = (size_t)ak_tiles_of(n_bytes, n_rows);
-    L.control = 0;
     L.state = 256;
     L.tile_row = L.state + ak_align(4 * tiles * 8);
-    size_t at = L.tile_row + ak_align(8 * (tiles * AKF_WARPS + 2));
-    L.scratch = at;
+    L.scratch = L.tile_row + ak_align(8 * (tiles * AKF_WARPS + 2));
     // Unigram row kernel / signatures: one 4-byte slot per code point (+ 2 per row)
-    size_t m = 4 * (size_t)(n_bytes + 2 * n_rows + 2);
-    // fast normalize: per-lane info words, tile totals / bases, slow work list
-    const size_t nf = ak_align(tiles * AK_BLOCK * 4) + ak_align(tiles * AKF_WARPS * 4) + ak_align((tiles * AKF_WARPS + 1) * 8) +
-                      ak_align((tiles * AK_BLOCK / 16 + 1024) * sizeof(AkSlowEntry));
-    if (nf > m) m = nf;
-    // segment / word tokenizers: warp-tile row table, two counts and two bases per 960-byte warp tile
-    const size_t n_wt = (size_t)n_bytes / AKN3_WARP_BYTES + 3;
-    const size_t sg = ak_align((2 * n_wt + 3) * 8) + 2 * ak_align(n_wt * 4) + 2 * ak_align(n_wt * 8);
-    if (sg > m) m = sg;
-    const size_t tok = ak_tok_ws(n_bytes, n_rows).total;
-    if (tok > m) m = tok;
-    L.total = at + ak_align(m);
+    const size_t rows = 4 * (size_t)(n_bytes + 2 * n_rows + 2);
+    const size_t n_wt = (size_t)n_bytes / AKN3_WARP_BYTES + 3, n_wt_words = (size_t)n_bytes / AKT_WARP_BYTES + 3;
+    AkNfWork nf;
+    AkSegWs sg;
+    int64_t* wrow;
+    AkWtWs wt;
+    const size_t m = std::max({rows, ak_nf_ws(tiles, nullptr, nf), ak_seg_ws(n_wt, nullptr, sg), ak_seg_mask_ws(n_wt, nullptr, wrow),
+                               ak_wt_ws(n_wt_words, nullptr, wt), ak_tok_ws(n_bytes, n_rows).total});
+    L.total = L.scratch + ak_align(m);
     return L;
 }
 
@@ -334,39 +425,38 @@ struct AkCall {
     AkBatch B;
     AkWsLayout L;
     char* ws;
+    AkControl* K;          // the workspace's control block
     size_t ws_bytes;       // what the caller really passed: the temporary streams use everything beyond the fixed part
     cudaStream_t stream;
 };
 
-// validates the common arguments, clears the control block + result, fills AkBatch (tiles for `mode`)
+// validates the common arguments, clears the control block, the tile states and the result, fills AkBatch (tiles for
+// `mode`).  The workspace is laid out for the larger of the text and layout_bytes: a fused call passes the capacity of
+// the normalized text its second stage reads.
 static int ak_begin(akshar_ctx* ctx, const uint8_t* d_text, const int64_t* d_row_offsets, int64_t n_rows, int64_t text_begin,
-                    int64_t text_end, int mode, int rows_block, int64_t* d_result, void* d_workspace, size_t workspace_bytes,
-                    void* stream, AkCall& C) {
+                    int64_t text_end, int64_t layout_bytes, int mode, int rows_block, int64_t* d_result, void* d_workspace,
+                    size_t workspace_bytes, void* stream, AkCall& C) {
     if (!ctx) return AKSHAR_E_ARG;
     if (!d_row_offsets || !d_result || n_rows < 0 || text_end < text_begin || (!d_text && text_end > text_begin) ||
-        (mode != AKSHAR_MODE_TILES && mode != AKSHAR_MODE_ROWS)) {
-        ctx->err = "bad argument";
-        return AKSHAR_E_ARG;
-    }
+        (mode != AKSHAR_MODE_TILES && mode != AKSHAR_MODE_ROWS))
+        return ak_fail(ctx, AKSHAR_E_ARG, "bad argument");
     const int64_t n_bytes = text_end - text_begin;
     // positions inside a call are 32-bit (event records, tile-relative offsets) and a row index shares a 32-bit word with
     // three kind bits: larger inputs are fed as several calls (row ranges keep their absolute offsets: text_begin / text_end)
-    if (n_bytes >= AKSHAR_MAX_CALL_BYTES || n_rows >= AKSHAR_MAX_CALL_ROWS) {
-        ctx->err = "batch too large for one call: at most 4 GiB - 64 KiB of text and 2^29 - 1 rows; split it by row ranges";
-        return AKSHAR_E_ARG;
-    }
+    if (n_bytes >= AKSHAR_MAX_CALL_BYTES || n_rows >= AKSHAR_MAX_CALL_ROWS)
+        return ak_fail(ctx, AKSHAR_E_ARG,
+                       "batch too large for one call: at most 4 GiB - 64 KiB of text and 2^29 - 1 rows; split it by row ranges");
+    const int64_t lay = layout_bytes > n_bytes ? layout_bytes : n_bytes;
     C.ctx = ctx;
-    C.L = ak_ws_layout(n_bytes, n_rows);
-    if (!d_workspace || workspace_bytes < C.L.total) {
-        ctx->err = "workspace too small: need " + std::to_string(C.L.total) + " bytes";
-        return AKSHAR_E_WORKSPACE;
-    }
+    C.L = ak_ws_layout(lay, n_rows);
+    if (!d_workspace || workspace_bytes < C.L.total) return ak_ws_short(ctx, C.L.total);
     C.ws = (char*)d_workspace;
+    C.K = (AkControl*)C.ws;
     C.ws_bytes = workspace_bytes;
     C.stream = (cudaStream_t)stream;
     AK_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t tiles = (size_t)ak_tiles_of(n_bytes, n_rows);
-    AK_CUDA(ctx, cudaMemsetAsync(C.ws, 0, 256 + ak_align(4 * tiles * 8), C.stream));
+    const size_t tiles = (size_t)ak_tiles_of(lay, n_rows);
+    AK_CUDA(ctx, cudaMemsetAsync(C.ws, 0, C.L.tile_row, C.stream));
     AK_CUDA(ctx, cudaMemsetAsync(d_result, 0, 4 * sizeof(int64_t), C.stream));
     AkBatch& B = C.B;
     B.text = d_text;
@@ -378,7 +468,7 @@ static int ak_begin(akshar_ctx* ctx, const uint8_t* d_text, const int64_t* d_row
     if (rows_block > 0) B.n_tiles = (int)((n_rows + rows_block - 1) / rows_block);
     else if (mode == AKSHAR_MODE_TILES) B.n_tiles = (int)((n_bytes + 1 + AK_TILE - 1) / AK_TILE);
     else B.n_tiles = (int)((n_rows + AK_BLOCK - 1) / AK_BLOCK);
-    B.ticket = (int*)C.ws;
+    B.ticket = &C.K->ticket;
     B.state0 = (unsigned long long*)(C.ws + C.L.state);
     B.state1 = B.state0 + tiles;
     B.result = d_result;
@@ -414,12 +504,18 @@ static int ak_after_launch(akshar_ctx* ctx, const char* what) {
         e = cudaDeviceSynchronize();
         if (e != cudaSuccess) fprintf(stderr, "akshar_b200: kernel '%s' failed: %s\n", what, cudaGetErrorString(e));
     }
-    if (e != cudaSuccess) {
-        ctx->err = std::string(what) + " launch: " + cudaGetErrorString(e);
-        return AKSHAR_E_CUDA;
-    }
+    if (e != cudaSuccess) return ak_fail(ctx, AKSHAR_E_CUDA, std::string(what) + " launch: " + cudaGetErrorString(e));
     ctx->launches++;
     return AKSHAR_OK;
+}
+
+// exclusive prefix sums of the n int32 counts v into base, their sum into *total (ak_scan.cuh), status bits into result[2].
+// With n_dyn the count is only known on the device and n bounds it.  Each scan of a call has its own ticket and tile states.
+static int ak_scan_counts(akshar_ctx* ctx, cudaStream_t s, const char* what, const int32_t* v, long long n, const long long* n_dyn,
+                          int64_t* base, int64_t* total, int* ticket, unsigned long long* state, int64_t* result) {
+    ak_scan_counts_kernel<<<ak_grid(ctx, 4, (int)(n / AKS_TILE + 1)), AKS_THREADS, 0, s>>>(v, n_dyn ? 0 : n, n_dyn, 1, base, total, ticket,
+                                                                                          state, (unsigned int*)&result[2]);
+    return ak_after_launch(ctx, what);
 }
 
 // a batch with no rows: every ragged output is just splits[0] = 0
