@@ -30,7 +30,7 @@ SYMBOLS = (
     'akshar_encode_bpe_batch', 'akshar_encode_unigram_batch', 'akshar_tokenizer_encode_batch', 'akshar_tokenizer_encode_batch_ex',
     'akshar_launch_count', 'akshar_timing_enable', 'akshar_timing_read', 'akshar_word_cache_hold', 'akshar_word_cache_stats', 'akshar_word_tokenize_batch', 'akshar_decode_workspace_bytes', 'akshar_decode_batch', 'akshar_composition_batch', 'akshar_merge_workspace_bytes', 'akshar_merge_clusters_batch', 'akshar_lines_workspace_bytes', 'akshar_lines_batch', 'akshar_join_rows', 'akshar_normalize_segment_batch',
     'akshar_windows_workspace_bytes', 'akshar_windows_count', 'akshar_windows_write', 'akshar_pair_windows_count',
-    'akshar_pair_windows_write', 'akshar_pack_workspace_bytes', 'akshar_pack_count', 'akshar_pack_write',
+    'akshar_pair_windows_write', 'akshar_pack_workspace_bytes', 'akshar_pack_count', 'akshar_pack_write', 'akshar_mlm_mask',
 )
 
 _lib = None
@@ -89,6 +89,7 @@ def load():
     L.akshar_pack_count.argtypes = [vp, vp, i32, vp, i64, vp, vp, i64, i64, i64, vp, vp, sz, vp]
     L.akshar_pack_write.argtypes = [vp, vp, i32, vp, i64, vp, vp, i64, i64, i64, i64, i64, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp,
                                     sz, vp]
+    L.akshar_mlm_mask.argtypes = [vp, i32, vp, i64, i64, c.c_uint64, u32, c.c_uint64, c.POINTER(c.c_uint64), i64, i64, vp, vp]
     L.akshar_load_bpe_json.argtypes = [vp, c.c_char_p, sz]
     L.akshar_load_spm_model.argtypes = [vp, c.c_char_p, sz]
     L.akshar_vocab_size.argtypes = [vp, i32]

@@ -62,6 +62,24 @@ def _ids_int32(v):
     return v.to(torch.int32)
 
 
+def mlm_thresholds(mlm_probability, mask_replace_prob, random_replace_prob):
+    """the three integer thresholds of akshar_mlm_mask (include/akshar_b200.h) for the collator's probabilities p, m, r:
+    t(q) = min(2^32, ceil(fl32(q) 2^32)), fl32 the rounding to float32 the collator's probability matrices get; t1 = t(p),
+    t2 = t(m), t3 = t(r / (1 - m)) with the ratio in double, or 0 when m = 1 or r = 0 (the collator's early return)"""
+    import math
+    import struct
+
+    def t(q):
+        return min(1 << 32, math.ceil(struct.unpack('<f', struct.pack('<f', q))[0] * 2 ** 32))
+    m, r = mask_replace_prob, random_replace_prob
+    return t(mlm_probability), t(m), 0 if m == 1 or r == 0 else t(r / (1 - m))
+
+
+def _check_uint(name, v, bits):
+    if isinstance(v, bool) or not isinstance(v, int) or not 0 <= v < 1 << bits:
+        raise ValueError('%s must be an int in [0, 2^%d)' % (name, bits))
+
+
 class BatchStatusError(RuntimeError):
     def __init__(self, bits, what):
         self.bits = bits
@@ -108,6 +126,7 @@ class Engine:
         self._ws = None
         self._vocab = {}
         self._pad = {}
+        self._mask = {}
 
     def __del__(self):
         try:
@@ -422,6 +441,14 @@ class Engine:
             self._pad[kind] = next((i for i, (p, t) in enumerate(self.vocab(kind)[1]) if p == '<pad>' and t == want), None)
         return self._pad[kind]
 
+    def mask_id(self, kind):
+        """id of the model's mask piece: the '<mask>' special token of a BPE model, the '<mask>' control piece of a
+        SentencePiece model; None without one"""
+        if kind not in self._mask:
+            want = 1 if kind == 0 else 3                          # BPE special token / SentencePiece CONTROL piece
+            self._mask[kind] = next((i for i, (p, t) in enumerate(self.vocab(kind)[1]) if p == '<mask>' and t == want), None)
+        return self._mask[kind]
+
     def windows_batch(self, ids, kind, max_length=None, padding='longest', truncation=False, stride=0,
                       return_overflowing_tokens=False, pad_to_multiple_of=None, padding_side='right', truncation_side='right',
                       pad_id=None, pair_ids=None):
@@ -609,6 +636,54 @@ class Engine:
             batch['cu_seq_lens_q'] = batch['cu_seq_lens_k'] = cu
             batch['max_length_q'] = batch['max_length_k'] = longest
         return batch, Ragged(rest_ids, rest_splits)
+
+    # ------------------------------------------------------------------ dense batches -> masked language-model batches
+    def mlm_mask(self, input_ids, kind, seed, mlm_probability=0.15, mask_replace_prob=0.8, random_replace_prob=0.1, epoch=0,
+                 row_base=0, mask_id=None, pad_id=None):
+        """transformers' DataCollatorForLanguageModeling(mlm=True) masking of a dense batch on the device: of the positions
+        that do not hold a special id of model `kind` (or pad_id), mlm_probability are selected; of those,
+        mask_replace_prob become mask_id (default: the model's '<mask>'), random_replace_prob of the rest a random id in
+        [0, vocabulary size), the others stay (the rule: include/akshar_b200.h, akshar_mlm_mask).  The draws are keyed by
+        (seed, epoch, row_base + row, position), so masking rows [a, b) with row_base = a gives rows a..b of the one-call
+        result, whatever the batch is cut into, padded to or spread over.
+        input_ids: contiguous int64 [N, L] on this engine's device (windows_batch / pack_batch output), changed in place.
+        -> (input_ids, labels): labels int64 [N, L], the original id where selected, else -100.
+        Raises ValueError for what the collator's __post_init__ refuses, a model without '<mask>' and no mask_id, seed /
+        row_base outside [0, 2^64), epoch outside [0, 2^32), and any other input_ids.  One kernel, no synchronisation."""
+        if mlm_probability is None or mlm_probability < 0 or mlm_probability > 1:
+            raise ValueError('mlm_probability should be between 0 and 1.')
+        if mask_replace_prob + random_replace_prob > 1:
+            raise ValueError('The sum of mask_replace_prob and random_replace_prob should not exceed 1')
+        if mask_replace_prob < 0 or mask_replace_prob > 1:
+            raise ValueError('mask_replace_prob should be between 0 and 1.')
+        if random_replace_prob < 0 or random_replace_prob > 1:
+            raise ValueError('random_replace_prob should be between 0 and 1.')
+        _check_uint('seed', seed, 64)
+        _check_uint('epoch', epoch, 32)
+        _check_uint('row_base', row_base, 64)
+        if mask_id is None:
+            mask_id = self.mask_id(kind)
+            if mask_id is None:
+                raise ValueError('This tokenizer does not have a mask token which is necessary for masked language modeling: '
+                                 'pass mask_id')
+        _check_uint('mask_id', mask_id, 63)
+        if pad_id is not None:
+            _check_uint('pad_id', pad_id, 63)
+        if not (isinstance(input_ids, torch.Tensor) and input_ids.dtype == torch.int64 and input_ids.dim() == 2 and
+                input_ids.is_contiguous() and input_ids.device == self.device):
+            raise ValueError('input_ids must be a contiguous int64 [N, L] tensor on %s' % self.device)
+        n, width = input_ids.shape
+        if row_base + n > 1 << 64:
+            raise ValueError('row_base + N must not exceed 2^64')
+        labels = torch.empty_like(input_ids)
+        t = (ctypes.c_uint64 * 3)(*mlm_thresholds(mlm_probability, mask_replace_prob, random_replace_prob))
+        rc = self.lib.akshar_mlm_mask(self._h, kind, input_ids.data_ptr(), n, width, seed, epoch, row_base, t, mask_id,
+                                      -1 if pad_id is None else pad_id, labels.data_ptr(), self._stream())
+        if rc == C.E_ARG:
+            raise ValueError(self.lib.akshar_last_error(self._h).decode())
+        if rc != 0:
+            self._err(rc, 'akshar_mlm_mask')
+        return input_ids, labels
 
     def segment_masks(self, batch, clusters=True, matras=False, runs=False, out=None, check=True):
         """segment_batch with AKSHAR_SEG_MASK: the boundaries as bit masks, one bit per text byte (bit p - begin set when a
@@ -800,6 +875,7 @@ class Engine:
             self._err(rc, 'akshar_load_bpe_json')
         self._vocab.pop(0, None)
         self._pad.pop(0, None)
+        self._mask.pop(0, None)
 
     def load_spm(self, path_or_bytes):
         """SentencePieceProcessor.Load for the CUDA path (reference tokenizer.py:88-91)"""
@@ -809,6 +885,7 @@ class Engine:
             self._err(rc, 'akshar_load_spm_model')
         self._vocab.pop(1, None)
         self._pad.pop(1, None)
+        self._mask.pop(1, None)
 
     def vocab(self, kind):
         """[(token str, type)] by id; kind 0 BPE, 1 Unigram"""

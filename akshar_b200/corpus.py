@@ -184,18 +184,27 @@ def encode_lines(tokenizer, input_file, as_device=False, chunk_bytes=CHUNK_BYTES
     return out
 
 
-def pack_lines(tokenizer, input_file, block_size, chunk_bytes=CHUNK_BYTES, **kwargs):
+def pack_lines(tokenizer, input_file, block_size, chunk_bytes=CHUNK_BYTES, mlm=None, **kwargs):
     """generator of packed causal-LM batches of a text file, one per piece of the file: every non-empty stripped line is
     a document, encoded on the device and packed by Engine.pack_batch (keywords: eos_id, separator_id,
     return_position_ids, return_seq_idx, return_flash_attn_kwargs).  The rest of each piece is the carry of the next,
     so the blocks are those of packing the whole file in one call.  The ids after the file's last whole block are
-    dropped, as transformers' run_clm.py `group_texts` drops them."""
+    dropped, as transformers' run_clm.py `group_texts` drops them.
+    mlm: a dict of Engine.mlm_mask keywords (seed, mlm_probability, mask_replace_prob, random_replace_prob, epoch,
+    mask_id, pad_id); every batch is then masked for masked-LM training, its labels replaced by the masked-LM ones, with
+    row_base = the blocks yielded before it, so that the masks are those of masking the one-call batch."""
     if tokenizer.model is None:
         raise ValueError("need model for IDs")
     if 'carry' in kwargs:
         raise ValueError('pack_lines threads the carry itself')
+    if mlm is not None and (not isinstance(mlm, dict) or 'row_base' in mlm):
+        raise ValueError('mlm must be a dict of mlm_mask keywords without row_base: pack_lines threads the row_base itself')
     carry = None
+    row_base = 0
     for rows in stream_rows(input_file, tokenizer._device, chunk_bytes):
         ids, _ = tokenizer.encode_batch(rows, as_device=True)
         batch, carry = tokenizer._eng.pack_batch(ids, block_size, carry=carry, **kwargs)
+        if mlm is not None:
+            batch['labels'] = tokenizer._eng.mlm_mask(batch['input_ids'], tokenizer.model.kind, row_base=row_base, **mlm)[1]
+            row_base += batch['input_ids'].shape[0]
         yield batch

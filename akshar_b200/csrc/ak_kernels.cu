@@ -42,6 +42,7 @@
 #include "ak_win_kernels.cuh"
 #include "ak_pair_kernels.cuh"
 #include "ak_pack_kernels.cuh"
+#include "ak_mlm_kernels.cuh"
 
 // ================================================================================================
 // host side: context, model upload, C ABI
@@ -70,6 +71,8 @@ struct akshar_ctx {
     // event-stream encoders (ak_tok.cuh): one word cache per model, image built at load
     AkcTable tok_cache[2];
     AkDecTable dec[2][2] = {};     // [kind][form]: piece tables of the on-device decode / detokenize (ak_decode.cuh)
+    const uint32_t* mlm_special[2] = {};  // [kind]: one bit per id of the model's special ids (akshar_mlm_mask)
+    int64_t mlm_bits[2] = {0, 0};
     bool uni_fast = false;         // the Unigram model has the shape the word-wise path needs
     int occ_words[2] = {0, 0}, occ_resolve[2] = {0, 0}, occ_check = 0, occ_emit = 0;
     // optional CUDA-event timing of the dominant kernel of each stage (bench.py's roofline line)

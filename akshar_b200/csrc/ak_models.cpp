@@ -251,6 +251,8 @@ std::string ak_parse_bpe_json(const char* json, size_t len, AkBpeHost& out) {
                 }
                 if (c->str.empty() || c->str.size() > 255) return "tokenizer JSON: bad added_tokens content";
                 specials.emplace_back(c->str, id);
+                const JVal* sp = a.get("special");
+                if (sp && sp->kind == JVal::Bool && sp->b) out.special_ids.push_back(id);
                 if (id > max_id) max_id = id;
             }
     }

@@ -26,6 +26,7 @@ struct AkBpeHost {
     std::vector<uint8_t> sp_bytes;
     std::vector<uint16_t> sp_off;                  // [n + 1]
     std::vector<int32_t> sp_ids;
+    std::vector<int32_t> special_ids;              // the added tokens marked "special": true
     int64_t n_merges = 0;
     int vocab_size = 0;
 };

@@ -180,6 +180,30 @@ class aksharTokenizer:
         ids, _ = self.encode_batch(texts, as_device=True)
         return self._eng.pack_batch(ids, block_size, **kwargs)
 
+    def encode_batch_mlm(self, texts, seed, block_size=None, text_pair=None, mlm_probability=0.15, mask_replace_prob=0.8,
+                         random_replace_prob=0.1, epoch=0, row_base=0, **kwargs):
+        """encode() over a batch, masked for masked-LM training as transformers' run_mlm.py batches it, in one of its two
+        modes.  Without block_size: encode_batch_tensors(texts, text_pair, **kwargs) followed by Engine.mlm_mask (the
+        window index is the row; the pad id of the windows is special) -> that dict with `labels` added.  With
+        block_size: encode_batch_packed(texts, block_size, **kwargs) followed by Engine.mlm_mask (the block index is the
+        row) -> (batch, rest) with the causal-LM labels replaced by the masked-LM ones; position_ids, seq_idx and
+        cu_seq_lens stay.  seed, the probabilities, epoch and row_base are those of Engine.mlm_mask."""
+        if self.model is None:
+            raise ValueError("need model for IDs")
+        mlm = dict(seed=seed, mlm_probability=mlm_probability, mask_replace_prob=mask_replace_prob,
+                   random_replace_prob=random_replace_prob, epoch=epoch, row_base=row_base)
+        if block_size is None:
+            batch = self.encode_batch_tensors(texts, text_pair, **kwargs)
+            pad = kwargs.get('pad_id')
+            pad = self._eng.pad_id(self.model.kind) if pad is None else pad
+            batch['labels'] = self._eng.mlm_mask(batch['input_ids'], self.model.kind, pad_id=pad, **mlm)[1]
+            return batch
+        if text_pair is not None:
+            raise ValueError('text_pair is not taken with block_size: packed blocks hold single texts')
+        batch, rest = self.encode_batch_packed(texts, block_size, **kwargs)
+        batch['labels'] = self._eng.mlm_mask(batch['input_ids'], self.model.kind, **mlm)[1]
+        return batch, rest
+
     def encode_batch_host(self, h_data, h_offsets, out_ids=None, out_splits=None, compact=False):
         """encode() over a batch given as pinned host tensors (uint8 text, int64 row offsets) -> pinned host tensors
         (int32 ids, int64 row_splits), or with compact=True a `CompactIds` (uint16 ids, int32 chunk-relative splits: a third

@@ -354,6 +354,34 @@ int akshar_pack_write(akshar_ctx* ctx, const void* d_ids, int ids_u16, const int
                       int64_t* d_labels, int64_t* d_position_ids, int32_t* d_seq_idx, int32_t* d_cu_seq_lens,
                       int32_t* d_rest_ids, int64_t* d_rest_splits, void* d_workspace, size_t workspace_bytes, void* stream);
 
+/* Masked language-model batches: transformers' DataCollatorForLanguageModeling(mlm=True) `torch_mask_tokens` over a dense
+ * batch, with its draws keyed by (seed, epoch, row, position), so that the masks do not depend on how a corpus is cut
+ * into calls, padded or spread over GPUs.
+ * In: d_input_ids int64 [n_rows, width] (as akshar_windows_write / akshar_pair_windows_write / akshar_pack_write write
+ * it), model `kind`, seed in [0, 2^64), epoch in [0, 2^32), row_base >= 0, the thresholds t1 t2 t3 (each <= 2^32), mask_id
+ * in [0, V), pad_id (-1: none).  V = the model's vocabulary size (akshar_vocab_size).
+ *   1. Special ids: the model's own (BPE: the added tokens marked "special": true; SentencePiece: the UNKNOWN and CONTROL
+ *      pieces) and pad_id: the collator's get_special_tokens_mask(already_has_special_tokens=True).  Other ids, those
+ *      outside [0, V) included, are not special.
+ *   2. Draws: one Philox4x32-10 block (Random123 / cuRAND Philox) per position: key (seed mod 2^32, seed >> 32),
+ *      counter (j, R mod 2^32, R >> 32, epoch) with R = row_base + n the row and j the position; its words are
+ *      (u_select, u_mask, u_random, r_id).
+ *   3. Thresholds, computed by the caller from the collator's probabilities p, m, r: t(q) = min(2^32, ceil(fl32(q) 2^32)),
+ *      fl32 = rounding to float32 (the collator's probability matrices are float32); t1 = t(p), t2 = t(m), t3 =
+ *      t(r / (1 - m)) with the ratio in double, and t3 = 0 when m = 1 or r = 0 (the collator returns before its third
+ *      draw).  u < t means drawn: u / 2^32 < fl32(q), what torch.bernoulli decides from a uniform u / 2^32.
+ *   4. Per position: selected = not special and u_select < t1; replaced = selected and u_mask < t2; random = selected,
+ *      not replaced and u_random < t3.
+ *   5. d_labels int64 [n_rows, width] = the original id where selected, else -100; d_input_ids, in place: mask_id where
+ *      replaced, floor(r_id V / 2^32) where random.  The random id is a multiply-high, not torch.randint's exactly
+ *      uniform draw: its relative bias is at most V / 2^32 (5.6e-6 for V = 24000).
+ * Refused with AKSHAR_E_ARG: a threshold above 2^32, width >= 2^32, mask_id outside [0, V), pad_id < -1, row_base +
+ * n_rows > 2^64; AKSHAR_E_NOMODEL when `kind` is not loaded.  n_rows = 0 or width = 0 launches nothing.  One kernel,
+ * no workspace, no synchronisation. */
+int akshar_mlm_mask(akshar_ctx* ctx, int kind, int64_t* d_input_ids, int64_t n_rows, int64_t width, uint64_t seed, uint32_t epoch,
+                    uint64_t row_base, const uint64_t thresholds[3], int64_t mask_id, int64_t pad_id, int64_t* d_labels,
+                    void* stream);
+
 /* Optional device-side timing of the dominant kernel of each stage, for roofline reporting: when enabled, the
  * library brackets that one launch with CUDA events on the caller's stream; akshar_timing_read waits for the
  * kernel and returns its duration of the most recent call. */
